@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — throughput of the EM hot path (E-step + M-step + model update) on synthetic planted-motif data.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|tiny] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|tiny] [--impl reference] [--dump-outputs DIR]
 
 A "step" is ONE EM iteration over the whole resident sequence set (E-step kernel, M-step accumulation kernel,
 count reduction + Motif::updateV + next odds table). Metric: bp.iter/s = (sum of input bases L0) x iterations /
@@ -14,6 +14,11 @@ JSON keys follow the driver's contract; extra objects:
   cpu_baseline  the reference's own EStep/MStep (oracle/_ref/ref_time, all host threads) on a bounded sample, rank 0, N=1
   e2e           same metric through the C ABI from HOST buffers: upload + index build + K iterations + model read-back
 `--impl reference` times only the CPU reference arm on the same workload definition (bounded sample per step).
+`--dump-outputs DIR` writes what the last timed step returned as DIR/<name>.npy, so that two builds can be compared output for
+output on the same seeded inputs. EM workloads: model (float32 v), counts (float32 n of the M-step), llh and vdiff (float32, one
+value each), r_sample (float32 posteriors of a fixed, seeded sample of sequences, one row each) and r_sample_seqs (float64 indices
+of those sequences). c4: zoops_pos / zoops_neg (float32 ZOOPS scores), argmax_pos / argmax_neg (float64 arg-max positions) and
+rows_pos / rows_neg (float64 rows of the scored subsets they belong to; a seeded sample above one million rows per set).
 """
 import argparse
 import hashlib
@@ -29,6 +34,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ in the source tree, which may be read-only; outputs go to --dump-outputs DIR / temp dirs
 
 from bammmotif2_b200 import synth  # noqa: E402
 from bammmotif2_b200 import hostmodel  # noqa: E402
@@ -42,7 +48,7 @@ Q = 0.3   # reference default prior (Global.cpp:52)
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 10); c5 and c4 --full time one whole CLI run instead")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--workload", default="c3", choices=sorted(synth.WORKLOADS))
     ap.add_argument("--nseq", type=int, default=0, help="override sequences per GPU (debug)")
@@ -56,7 +62,60 @@ def parse_args():
     ap.add_argument("--full", action="store_true", help="workload c4: the WHOLE --FDR run through the drop-in CLI (bin/BaMMmotif) instead of one fold's scoring")
     ap.add_argument("--no-strong", action="store_true", help="N > 1: skip the strong-scaling run (one set split over the ranks)")
     ap.add_argument("--cpu-sample", type=int, default=0, help="sequences in the CPU sample (default by workload)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)")
+    args = ap.parse_args()
+    whole_run = args.workload == "c5" or (args.workload == "c4" and args.full)
+    if whole_run and args.steps is not None:
+        ap.error("--steps does not apply to --workload c5 or c4 --full: they time one whole command-line run")
+    if args.steps is None:
+        args.steps = 10
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or whole_run):
+        ap.error("--dump-outputs writes the outputs of the timed device path (--workload c2, c3, tiny or c4 without --full)")
+    return args
+
+
+DUMP_SAMPLE_SEQS = 1024
+DUMP_SAMPLE_BYTES = 32 << 20
+DUMP_SCORES_PER_SET = 1_000_000
+
+
+def dump_scores(out_dir, pos, neg):
+    """c4: the ZOOPS scores (float32) and arg-max positions (float64) a caller of the timed step receives for the positive and
+    the negative subset, each with the subset rows they belong to (float64); a set above DUMP_SCORES_PER_SET is a seeded sample."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (zoops, z) in (("pos", pos), ("neg", neg)):
+        rows = np.arange(len(zoops))
+        if len(rows) > DUMP_SCORES_PER_SET:
+            rows = np.sort(np.random.default_rng(0).choice(len(rows), size=DUMP_SCORES_PER_SET, replace=False))
+        np.save(os.path.join(out_dir, "zoops_%s.npy" % name), zoops[rows].astype(np.float32))
+        np.save(os.path.join(out_dir, "argmax_%s.npy" % name), z[rows].astype(np.float64))
+        np.save(os.path.join(out_dir, "rows_%s.npy" % name), rows.astype(np.float64))
+
+
+def dump_outputs(out_dir, em):
+    """Writes the arrays a caller of the timed loop receives after its last iteration (bamm_em_iterate's llh / sum|dv|,
+    bamm_em_get_model, bamm_em_get_counts, bamm_em_get_r) as float32 / float64 .npy files; r only for a seeded sample of
+    sequences (every sequence of a bench set has the same length, so the sample is one row per sequence).
+    Call it after the loop timings have been read: em.iterate(0) re-reads the last iteration's scalars and resets the timings."""
+    from bammmotif2_b200 import capi
+    os.makedirs(out_dir, exist_ok=True)
+    llh, vdiff = em.iterate(0)
+    nseq = em.nsub
+    rsize = int(capi.load().bamm_em_r_size(em.h))
+    assert rsize % nseq == 0, "sequences of unequal length"
+    per_seq = rsize // nseq
+    n = max(1, min(nseq, DUMP_SAMPLE_SEQS, DUMP_SAMPLE_BYTES // (4 * per_seq)))
+    seqs = np.sort(np.random.default_rng(0).choice(nseq, size=n, replace=False))
+    r = np.empty((n, per_seq), np.float32)
+    for i, s in enumerate(seqs):
+        capi._check(capi.load().bamm_em_get_r(em.h, int(s), 1, r[i].ctypes.data_as(capi._f32p)))
+    arrays = {"model": em.model(), "counts": em.counts(), "llh": np.array([llh], np.float32), "vdiff": np.array([vdiff], np.float32),
+              "r_sample": r, "r_sample_seqs": seqs.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -541,6 +600,8 @@ def run_c4(args, wl):
     torch.cuda.synchronize()
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_scores(args.dump_outputs, out_pos, out_neg)
     if world > 1:
         t = torch.tensor([kernel_ms, wall], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -777,6 +838,8 @@ def main():
     llh_after = None
     if world == 1:
         llh_after = em.iterate(0)[0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, em)
 
     # ---- strong scaling: ONE set of wl["nseq"] sequences (rank 0's data) split into contiguous blocks over the ranks -----------
     strong = None
