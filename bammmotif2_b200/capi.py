@@ -62,6 +62,7 @@ SIGNATURES = {
     "bamm_em_set_exchange_buffer": (C.c_int, [_vp, _vp, C.c_uint64]),
     "bamm_em_launch_count": (C.c_int, [_vp, _u64p]),
     "bamm_em_estep_info": (C.c_int, [_vp, _u64p]),
+    "bamm_em_bound_reuse_info": (C.c_int, [_vp, _u64p, C.POINTER(C.c_float)]),
     "bamm_em_destroy": (None, [_vp]),
     "bamm_em_exchange_buffer": (C.c_int, [_vp, C.POINTER(_vp), _u64p]),
     "bamm_em_set_global_nseq": (C.c_int, [_vp, C.c_uint64]),
@@ -418,6 +419,14 @@ class EM:
         _check(load().bamm_em_estep_info(self.h, a))
         return dict(pruned=bool(a[0]), G=int(a[1]), G_bound=int(a[2]), dense_ran=bool(a[3]), candidates=int(a[4]), active=int(a[5]),
                     passes=int(a[6]), plain_smem=bool(a[7]))
+
+    def bound_reuse_info(self):
+        """Bound reuse of the pruned E-step (bamm_em_bound_reuse_info): dict(enabled, full, watch, watched, last_watch, valid, log2_drift)."""
+        a = (C.c_uint64 * 6)()
+        d = C.c_float(0.0)
+        _check(load().bamm_em_bound_reuse_info(self.h, a, C.byref(d)))
+        return dict(enabled=bool(a[0]), full=int(a[1]), watch=int(a[2]), watched=int(a[3]), last_watch=bool(a[4]), valid=bool(a[5]),
+                    log2_drift=float(d.value))
 
     def set_exchange_buffer(self, dev_ptr, words):
         _check(load().bamm_em_set_exchange_buffer(self.h, _vp(dev_ptr), words))

@@ -201,6 +201,15 @@ struct bamm_em {
     float* d_mask_part = nullptr;    // column passes: partial product per masked window of every sequence (k_emasked)
     ulonglong2* d_seqacc = nullptr;  // per list sequence: normaliser terms of its masked windows (k_emasked -> k_eexact)
     uint32_t* d_eflags = nullptr;   // CandList::flags (8 words)
+    // bound reuse (CandList::went ..): watch list, its region offsets and per-sequence records, the tables it was built from,
+    // the device-side state (BREUSE_WORDS); d_reuse == nullptr: off (BAMM_NO_BOUND_REUSE, or no memory for the list)
+    uint32_t* d_watch = nullptr; uint64_t* d_wreg_off = nullptr; uint2* d_watch_seq = nullptr;
+    float* d_btab_ref = nullptr; uint32_t* d_reuse = nullptr;
+    int bound_slack = 10;           // m: the watch list holds the windows whose bound reaches thr 2^-m (BAMM_BOUND_SLACK)
+    // BAMM_DEBUG_BOUND (capi_em.inl, debug_bound): pruned E-steps since set_model, bound tables of the previous / first / third one
+    int dbg_estep = 0;
+    std::vector<uint32_t> dbg_tab_prev, dbg_tab_1, dbg_tab_3;
+    unsigned long long* d_dbg_hist = nullptr;
     bool r_mat = true;          // d_r holds the posteriors of the last E-step (false after a pruned E-step until bamm_em_get_r)
     const float *d_s_e = nullptr, *d_sT_e = nullptr, *d_tab_e = nullptr;   // the tables the last E-step read
     float q_e = 0.3f;           // ... and its prior

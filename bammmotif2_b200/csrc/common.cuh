@@ -115,7 +115,22 @@ struct CandList {
     uint32_t* flags;          // [0] != 0: this iteration runs the dense E-step (a region overflowed, or the hold below is active)
                               // [1] iterations the dense E-step stays switched on after an overflow; [2..3] 64-bit candidate count (diagnostics)
                               // [4] length of the current hold; [5] != 0: a region overflowed in the last E-step (k_estep_begin turns it into a hold)
+    // bound reuse (k_ebound_watch): the full pass also lists the windows whose bound reaches thr * watch_scale (the watch list,
+    // same region layout and order as the candidates); while the tables have not moved far enough from those it was built from
+    // (tab_ref) to lift any other window to thr, only the listed windows are bounded again. reuse == nullptr: always full passes.
+    uint32_t* went;           // watched window starts
+    const uint64_t* wreg_off; // [nregions+1] first entry of every watch region
+    uint2* wseq;              // [nlist] (first entry inside the region, count)
+    uint32_t* reuse;          // BREUSE_WORDS words, see below
+    float* tab_ref;           // the bound tables the watch list was built from (copied by CTA 0 of the full pass)
+    float watch_scale;        // 2^-m, m = slack in bits
 };
+// words of CandList::reuse. [BR_MODE] this E-step runs 0: the full pass and rebuilds the watch list, 1: the watch pass, 2: the full
+// pass without the list (the last one was too long to pay); [BR_SKIP] full passes that kept a too long list; [BR_WFULL] a watch region filled up in the last list build; [BR_VALID] the watch list matches tab_ref and q_ref;
+// [BR_QREF] q of the full pass that built it (float bits); [BR_LAMBDA] log2 of the last drift bound (float bits);
+// [BR_FULL], [BR_WATCH] passes of each kind (diagnostics); [BR_WCOUNT] entries of the watch list;
+// [BR_RHO + g] max_e B_g[e] / tab_ref_g[e] of the tables built since the last E-step (float bits, k_make_bound_tables)
+constexpr int BR_MODE = 0, BR_VALID = 1, BR_QREF = 2, BR_LAMBDA = 3, BR_FULL = 4, BR_WATCH = 5, BR_WCOUNT = 6, BR_SKIP = 7, BR_WFULL = 8, BR_RHO = 9, BREUSE_WORDS = BR_RHO + MAXG;
 // After an overflow the dense E-step runs for 2 iterations, then the bound pass tries again; every further overflow in a row
 // doubles the hold (a model whose posteriors stay diffuse pays log2(iterations) wasted bound passes, one that sharpens after
 // the first iterations is back on the pruned path at once); a pruned iteration that fits resets it.

@@ -318,9 +318,12 @@ k_ebound(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __res
     extern __shared__ __align__(16) float tab[];
     __shared__ unsigned long long stage_bar;
     volatile uint32_t* flags = cl.flags;
-    if (flags[0] != 0u) return;
+    if (flags[0] != 0u || (cl.reuse != nullptr && cl.reuse[BR_MODE] == 1u)) return;
+    const bool build_list = cl.reuse != nullptr && cl.reuse[BR_MODE] == 0u;
     bulk_stage_begin(tab, tab_g, gp.table_bytes, &stage_bar);
     bulk_stage_wait(&stage_bar);
+    if (build_list && blockIdx.x == 0)                    // the tables this watch list is built from
+        for (uint32_t i = threadIdx.x; i < (gp.table_bytes >> 2); i += blockDim.x) cl.tab_ref[i] = tab[i];
     const int lane = threadIdx.x & 31;
     const uint32_t warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const uint32_t nwarps = gridDim.x * (blockDim.x >> 5);
@@ -331,6 +334,11 @@ k_ebound(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __res
     const uint32_t ccap = (uint32_t)(cl.reg_off[warp + 1] - cl.reg_off[warp]);
     uint32_t cpos = 0;
     bool ok = true;
+    // watch list: written in the same order as the candidates, so that filtering it keeps the candidates' order
+    bool wok = build_list;
+    uint32_t* __restrict__ wreg = wok ? cl.went + cl.wreg_off[warp] : nullptr;
+    const uint32_t wcap = wok ? (uint32_t)(cl.wreg_off[warp + 1] - cl.wreg_off[warp]) : 0u;
+    uint32_t wpos = 0;
     // a lane owns the windows 2 lane, 2 lane + 1 of every chunk of 64: one entry of a pair table bounds both
     const int lane_word = (2 * lane - KD) >> 4;
     const int sft = 2 * ((2 * lane - KD) & 15);
@@ -350,10 +358,11 @@ k_ebound(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __res
             const int L = (int)sq.L, LW1 = L - W + 1, mid = (int)sq.mid;
             // bound * q/LW1 >= thr0  <=>  bound >= thr0 LW1 / q (thr0 already carries the rounding margin of the bound)
             const float thr = gp.thr0 * (float)LW1 / gp.q;
+            const float thw = thr * cl.watch_scale;
             const int tl = min(max(L - 2 * W + 2, 0), LW1);
             int n0 = tl, n1 = tl;
             if (mid >= 0) { n0 = min(max(mid - W + 1, 0), tl); n1 = min(mid + K + 1, tl); }
-            const uint32_t start = cpos;
+            const uint32_t start = cpos, wstart = wpos;
             const int nch = (tl + 63) >> 6;
             uint32_t u0 = 0, u1 = 0, u2 = 0;
             // The hot loop only records, per lane, WHICH of its windows pass (bit c = window 2 lane + 64 c, bit 16 + c = the
@@ -364,7 +373,7 @@ k_ebound(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __res
                 const int ce = min(nch, cb + 16);
                 const bool last_block = ce == nch;
                 const int c_pf = last_block ? max(ce - 4, cb) : ce;      // chunk before which the next sequence's first words are requested
-                uint32_t mine = 0u, bit = 1u;
+                uint32_t mine = 0u, watched = 0u, bit = 1u;
                 auto chunk = [&]() {
                     const uint32_t whi = __funnelshift_l(t1, t0, sft), wlo = __funnelshift_l(t2, t1, sft);
                     wl += 4;
@@ -378,6 +387,8 @@ k_ebound(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __res
                     }
                     if (b0 >= thr) mine |= bit;
                     if (b1 >= thr) mine |= bit << 16;
+                    if (b0 >= thw) watched |= bit;
+                    if (b1 >= thw) watched |= bit << 16;
                     bit <<= 1;
                 };
 #pragma unroll 2
@@ -414,9 +425,28 @@ k_ebound(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __res
                     creg[at++] = (uint32_t)(pb + 64 * (b & 15) + (b >> 4));
                 }
                 cpos += total;
+                if (wok) {                                       // the same for the watch list; when it is full, only it is dropped
+                    watched &= keep;
+                    const uint32_t wcnt = __popc(watched);
+                    uint32_t winc = wcnt;
+#pragma unroll
+                    for (int o = 1; o < 32; o <<= 1) { const uint32_t v = __shfl_up_sync(FULL, winc, o); if (lane >= o) winc += v; }
+                    const uint32_t wtotal = __shfl_sync(FULL, winc, 31);
+                    if (wpos + wtotal > wcap) wok = false;
+                    else {
+                        uint32_t wat = wpos + winc - wcnt;
+                        while (watched) {
+                            const int b = __ffs(watched) - 1;
+                            watched &= watched - 1u;
+                            wreg[wat++] = (uint32_t)(pb + 64 * (b & 15) + (b >> 4));
+                        }
+                        wpos += wtotal;
+                    }
+                }
             }
             if (nch == 0) { const uint32_t* __restrict__ wn = pv.words + sq_next.word_off + lane_word; u0 = wn[0]; u1 = wn[1]; u2 = wn[2]; }
             if (lane == 0) cl.seq[li] = make_uint2(start, cpos - start);
+            if (wok && lane == 0) cl.wseq[li] = make_uint2(wstart, wpos - wstart);
             if (!ok || !more) break;
             li = li_next; sq = sq_next; n_next = n_nn;
             wl = pv.words + sq.word_off + lane_word;
@@ -425,6 +455,139 @@ k_ebound(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __res
     }
     if (!ok && lane == 0) { flags[5] = 1u; __threadfence(); flags[0] = 1u; }
     if (lane == 0 && cpos) atomicAdd(reinterpret_cast<unsigned long long*>(cl.flags + 2), (unsigned long long)cpos);
+    if (build_list && lane == 0) {
+        if (!wok || !ok) cl.reuse[BR_VALID] = 0u;     // an incomplete list (full watch region, or a warp that stopped early) is not used
+        if (!wok) cl.reuse[BR_WFULL] = 1u;
+        else if (wpos) atomicAdd(&cl.reuse[BR_WCOUNT], wpos);
+    }
+}
+
+// ---- pruned E-step, part 1 with reuse: bounds of the watched windows only -------------------------------------------
+// Runs instead of k_ebound when k_estep_begin found that no window outside the watch list can reach thr with the current tables.
+// Same warp -> sequence walk, same thr, same products (window p's bound is the low half of the entry at p's window word: the
+// value k_ebound reads from the low half at p or the high half at p-1), so the candidates come out as the full pass would list
+// them, in the same order: the watch list holds them in that order. A region overflows exactly when the full pass's would (its
+// warp has more candidates than slots), and then raises the same dense fall-back.
+template <int G1, bool FAST>
+__global__ void __launch_bounds__(BAMM_E_THREADS, 1)
+k_ebound_watch(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __restrict__ tab_g, CandList cl) {
+    extern __shared__ __align__(16) float tab[];
+    __shared__ unsigned long long stage_bar;
+    volatile uint32_t* flags = cl.flags;
+    if (flags[0] != 0u || cl.reuse == nullptr || cl.reuse[BR_MODE] != 1u) return;
+    bulk_stage_begin(tab, tab_g, gp.table_bytes, &stage_bar);
+    bulk_stage_wait(&stage_bar);
+    const int lane = threadIdx.x & 31;
+    const uint32_t warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const uint32_t nwarps = gridDim.x * (blockDim.x >> 5);
+    const int W = gp.W, KD = gp.kd;
+    const uint32_t tab_s = (uint32_t)__cvta_generic_to_shared(tab);
+    GroupConsts<G1> gc; load_consts<G1>(gc, gp, tab_s);
+    uint32_t lt_mask;
+    asm("mov.u32 %0, %%lanemask_lt;" : "=r"(lt_mask));
+    uint32_t* __restrict__ creg = cl.ent + cl.reg_off[warp];
+    const uint32_t ccap = (uint32_t)(cl.reg_off[warp + 1] - cl.reg_off[warp]);
+    const uint32_t* __restrict__ wreg = cl.went + cl.wreg_off[warp];
+    uint32_t cpos = 0;
+    bool ok = true;
+    uint32_t li = warp;
+    if (li < pv.nlist) {
+        PackedSeq sq = pv.seqs[pv.seq_ids[li]];
+        uint2 ws = cl.wseq[li];
+        uint32_t n_next = li + nwarps < pv.nlist ? pv.seq_ids[li + nwarps] : 0u;
+        for (;;) {
+            if (flags[0] != 0u) break;
+            const uint32_t li_next = li + nwarps;
+            const bool more = li_next < pv.nlist;
+            PackedSeq sq_next = sq;
+            uint2 ws_next = ws;
+            uint32_t n_nn = 0u;
+            if (more) { sq_next = pv.seqs[n_next]; ws_next = cl.wseq[li_next]; if (li_next + nwarps < pv.nlist) n_nn = pv.seq_ids[li_next + nwarps]; }
+            const int LW1 = (int)sq.L - W + 1;
+            const float thr = gp.thr0 * (float)LW1 / gp.q;
+            const uint32_t* __restrict__ wseq = pv.words + sq.word_off;
+            const uint32_t* __restrict__ wl = wreg + ws.x;
+            const uint32_t start = cpos;
+            uint32_t p_next = lane < ws.y ? wl[lane] : 0u;
+            for (uint32_t e0 = 0; e0 < ws.y; e0 += 32) {
+                const bool on = e0 + lane < ws.y;
+                const int p = (int)p_next;
+                if (e0 + 32 + lane < ws.y) p_next = wl[e0 + 32 + lane];      // next batch
+                uint32_t whi, wlo;
+                window_bits(wseq, p - KD, whi, wlo);
+                float b0 = 1.0f;
+#pragma unroll
+                for (int g = 0; g < G1; g++) {
+                    const float f0 = __uint_as_float(__float_as_uint(lds_f32(group_offset<G1, FAST>(gc, g, whi, wlo), gc.ab[g])) << 16);
+                    b0 = g ? b0 * f0 : f0;
+                }
+                const bool pass = on && b0 >= thr;
+                const uint32_t m = __ballot_sync(FULL, pass);
+                const uint32_t cnt = __popc(m);
+                if (cpos + cnt > ccap) { ok = false; break; }
+                if (pass) creg[cpos + __popc(m & lt_mask)] = (uint32_t)p;
+                cpos += cnt;
+            }
+            if (!ok) break;
+            if (lane == 0) cl.seq[li] = make_uint2(start, cpos - start);
+            if (!more) break;
+            li = li_next; sq = sq_next; ws = ws_next; n_next = n_nn;
+        }
+    }
+    if (!ok && lane == 0) { flags[5] = 1u; __threadfence(); flags[0] = 1u; }
+    if (lane == 0 && cpos) atomicAdd(reinterpret_cast<unsigned long long*>(cl.flags + 2), (unsigned long long)cpos);
+}
+
+// ---- diagnostic (BAMM_DEBUG_BOUND): distribution of the bounds relative to the candidate threshold ---------------------
+// Same windows, tables and products as k_ebound; instead of a list, a histogram of log2(b(p) / thr) in quarter bits
+// (bin BOUND_HIST_ZERO + floor(4 log2), clamped; bin 0 also takes b = 0). One shared-memory histogram per CTA, one flush.
+constexpr int BOUND_HIST_BINS = 512, BOUND_HIST_ZERO = 384;
+template <int G1, bool FAST>
+__global__ void __launch_bounds__(BAMM_E_THREADS, 1)
+k_ebound_hist(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __restrict__ tab_g, unsigned long long* __restrict__ hist) {
+    extern __shared__ __align__(16) float tab[];
+    __shared__ unsigned long long stage_bar;
+    __shared__ uint32_t h[BOUND_HIST_BINS];
+    for (int i = threadIdx.x; i < BOUND_HIST_BINS; i += blockDim.x) h[i] = 0u;
+    bulk_stage_begin(tab, tab_g, gp.table_bytes, &stage_bar);
+    bulk_stage_wait(&stage_bar);
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const uint32_t warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const uint32_t nwarps = gridDim.x * (blockDim.x >> 5);
+    const int W = gp.W, K = gp.K, KD = gp.kd;
+    const uint32_t tab_s = (uint32_t)__cvta_generic_to_shared(tab);
+    GroupConsts<G1> gc; load_consts<G1>(gc, gp, tab_s);
+    auto bin_of = [](float b, float thr) {
+        if (!(b > 0.0f)) return 0;
+        const int k = (int)floorf(4.0f * log2f(b / thr)) + BOUND_HIST_ZERO;
+        return min(max(k, 0), BOUND_HIST_BINS - 1);
+    };
+    for (uint32_t li = warp; li < pv.nlist; li += nwarps) {
+        const PackedSeq sq = pv.seqs[pv.seq_ids[li]];
+        const int L = (int)sq.L, LW1 = L - W + 1, mid = (int)sq.mid;
+        const float thr = gp.thr0 * (float)LW1 / gp.q;
+        const int tl = min(max(L - 2 * W + 2, 0), LW1);
+        int n0 = tl, n1 = tl;
+        if (mid >= 0) { n0 = min(max(mid - W + 1, 0), tl); n1 = min(mid + K + 1, tl); }
+        const uint32_t* __restrict__ wseq = pv.words + sq.word_off;
+        for (int c = 0; c < (tl + 63) >> 6; c++) {
+            const int p = 64 * c + 2 * lane;
+            uint32_t whi, wlo;
+            window_bits(wseq, p - KD, whi, wlo);
+            float b0 = 1.0f, b1 = 1.0f;
+#pragma unroll
+            for (int g = 0; g < G1; g++) {
+                const uint32_t e = __float_as_uint(lds_f32(group_offset<G1, FAST>(gc, g, whi, wlo), gc.ab[g]));
+                const float f0 = __uint_as_float(e << 16), f1 = __uint_as_float(e & 0xffff0000u);
+                b0 = g ? b0 * f0 : f0; b1 = g ? b1 * f1 : f1;
+            }
+            if (p < tl && (p < n0 || p >= n1)) atomicAdd(&h[bin_of(b0, thr)], 1u);
+            if (p + 1 < tl && (p + 1 < n0 || p + 1 >= n1)) atomicAdd(&h[bin_of(b1, thr)], 1u);
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < BOUND_HIST_BINS; i += blockDim.x) if (h[i]) atomicAdd(&hist[i], (unsigned long long)h[i]);
 }
 
 // ---- pruned E-step, part 0: the windows over the N and the truncated tail ----------------------------------------------

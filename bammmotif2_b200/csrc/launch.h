@@ -25,6 +25,11 @@ int launch_estep_bound(const EStepLaunch& l, bool optin_only, bool fast, const P
 int launch_estep_exact(const EStepLaunch& l, bool optin_only, bool fast, const PackedView* pv, const GroupPlan& gp, const float* d_tab,
                        const float* d_s, uint32_t plain_words, bool stage, const CandList* cl, const ulonglong2* d_seqacc,
                        float* d_partial, unsigned long long* d_scal, const ActiveList* al);
+// diagnostic (BAMM_DEBUG_BOUND): histogram of log2(bound / threshold) over the windows k_ebound bounds, added to d_hist
+// (estep_bound_hist_bins() 64-bit counters, quarter-bit bins, bin estep_bound_hist_zero() starts at bound = threshold)
+int launch_estep_bound_hist(const EStepLaunch& l, bool fast, const PackedView* pv, const GroupPlan& gp, const float* d_tab, unsigned long long* d_hist);
+int estep_bound_hist_bins();
+int estep_bound_hist_zero();
 // bytes of the per-warp staging buffers k_eexact appends to its shared memory when `stage` is set
 size_t estep_stage_bytes(int block);
 

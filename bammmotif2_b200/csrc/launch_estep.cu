@@ -33,8 +33,10 @@ int launch_estep_dense(const EStepLaunch& l, bool optin_only, bool fast, bool mu
 
 template <int G, bool FAST>
 static int bound_one(const EStepLaunch& l, bool optin_only, const PackedView* pv, const GroupPlan& gp, const float* d_tab, const CandList* cl) {
-    if (optin_only) return optin(k_ebound<G, FAST>, gp.table_bytes);
+    if (optin_only) return optin(k_ebound<G, FAST>, gp.table_bytes) || optin(k_ebound_watch<G, FAST>, gp.table_bytes);
+    // with bound reuse both kernels are launched; the device flag k_estep_begin set lets exactly one of them do the pass
     k_ebound<G, FAST><<<l.grid, l.block, gp.table_bytes, l.stream>>>(*pv, gp, d_tab, *cl);
+    if (cl->reuse) k_ebound_watch<G, FAST><<<l.grid, l.block, gp.table_bytes, l.stream>>>(*pv, gp, d_tab, *cl);
     return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 int launch_estep_bound(const EStepLaunch& l, bool optin_only, bool fast, const PackedView* pv, const GroupPlan& gp, const float* d_tab,
@@ -46,6 +48,23 @@ int launch_estep_bound(const EStepLaunch& l, bool optin_only, bool fast, const P
         default: return -1;
     }
 }
+
+template <int G, bool FAST>
+static int bound_hist_one(const EStepLaunch& l, const PackedView* pv, const GroupPlan& gp, const float* d_tab, unsigned long long* d_hist) {
+    if (optin(k_ebound_hist<G, FAST>, gp.table_bytes)) return -1;
+    k_ebound_hist<G, FAST><<<l.grid, l.block, gp.table_bytes, l.stream>>>(*pv, gp, d_tab, d_hist);
+    return cudaGetLastError() == cudaSuccess ? 0 : -1;
+}
+int launch_estep_bound_hist(const EStepLaunch& l, bool fast, const PackedView* pv, const GroupPlan& gp, const float* d_tab, unsigned long long* d_hist) {
+    switch (gp.G) {
+#define X(g) case g: return fast ? bound_hist_one<g, true>(l, pv, gp, d_tab, d_hist) : bound_hist_one<g, false>(l, pv, gp, d_tab, d_hist);
+        X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8)
+#undef X
+        default: return -1;
+    }
+}
+int estep_bound_hist_bins() { return BOUND_HIST_BINS; }
+int estep_bound_hist_zero() { return BOUND_HIST_ZERO; }
 
 size_t estep_stage_bytes(int block) { return (size_t)(block / 32) * STAGE_WORDS * sizeof(uint32_t); }
 

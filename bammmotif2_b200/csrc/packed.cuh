@@ -229,7 +229,10 @@ __device__ __forceinline__ uint32_t bf16_up(float x) {      // smallest bfloat16
     if (b & 0xffffu) b = (b | 0xffffu) + 1u;
     return b >> 16;
 }
-__global__ void k_make_bound_tables(const float* __restrict__ s, const float* __restrict__ U, BoundLevels bl, GroupPlan gp, uint32_t* __restrict__ tab) {
+// ref != nullptr (bound reuse): rho[g] = max over the group's bfloat16 values of new / ref, rounded up (+inf where ref is 0 and the new
+// value is not; a zero new value bounds nothing and is skipped): one atomicMax of the float bits per warp and group.
+__global__ void k_make_bound_tables(const float* __restrict__ s, const float* __restrict__ U, BoundLevels bl, GroupPlan gp, uint32_t* __restrict__ tab,
+                                    const uint32_t* __restrict__ ref, uint32_t* __restrict__ rho) {
     const uint32_t total = gp.table_bytes >> 2;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
         int g = 0;
@@ -249,10 +252,29 @@ __global__ void k_make_bound_tables(const float* __restrict__ s, const float* __
             packed |= bf16_up(p) << (16 * h);
         }
         tab[i] = packed;
+        if (ref) {
+            const uint32_t r = ref[i];
+            uint32_t x = 0u;
+            for (int h = 0; h < 2; h++) {
+                const float B = __uint_as_float(h ? packed & 0xffff0000u : packed << 16), R = __uint_as_float(h ? r & 0xffff0000u : r << 16);
+                const float q = B == 0.0f ? 0.0f : R == 0.0f ? __int_as_float(0x7f800000) : __fdiv_ru(B, R);
+                x = max(x, __float_as_uint(q));             // non-negative floats order as their bits
+            }
+            const uint32_t peers = __match_any_sync(__activemask(), g);
+            x = __reduce_max_sync(peers, x);
+            if ((__ffs(peers) - 1) == (int)(threadIdx.x & 31)) atomicMax(&rho[g], x);
+        }
     }
 }
-// start of an E-step: scalars and list-overflow flag cleared; the dense-hold counter of the pruned path ticks down
-__global__ void k_estep_begin(unsigned long long* __restrict__ scal, uint32_t* __restrict__ overflow, uint32_t* __restrict__ eflags) {
+// start of an E-step: scalars and list-overflow flag cleared; the dense-hold counter of the pruned path ticks down.
+// reuse != nullptr: choose between the full bound pass and the watch pass (k_ebound, k_ebound_watch). A window outside the watch
+// list has b_ref(p) < thr_ref 2^-m; the bounds now are at most P = prod_g rho_g times the reference ones, so b(p) < thr when
+// P thr_ref / thr < 2^m. thr = thr0 LW1 / q with thr0 proportional to 1 - q, so thr_ref / thr = ((1-q_ref)/q_ref) / ((1-q)/q).
+// Rounding: b(p) and b_ref(p) are float products of G1 <= 8 factors, each within (1+2^-24)^7 of the exact product, thr within
+// a few ulps; the factor 1 + 2^-16 in P covers all of it. Intermediate products that end up subnormal lose relative accuracy,
+// but their absolute error (< 2^-149 times the remaining factors, each < 2^64) stays far below thr * 2^-m (> 2^-80 for m <= 32).
+__global__ void k_estep_begin(unsigned long long* __restrict__ scal, uint32_t* __restrict__ overflow, uint32_t* __restrict__ eflags,
+                              uint32_t* __restrict__ reuse, float q, float slack_pow /* 2^m */, int G1, unsigned long long nwin) {
     if (threadIdx.x == 0) {
         scal[0] = 0ull; scal[1] = 0ull;
         if (overflow) *overflow = 0u;
@@ -266,6 +288,23 @@ __global__ void k_estep_begin(unsigned long long* __restrict__ scal, uint32_t* _
             eflags[0] = hold ? 1u : 0u;
             eflags[1] = hold ? hold - 1u : 0u;
             eflags[2] = 0u; eflags[3] = 0u;
+        }
+        if (reuse) {
+            const float qr = __uint_as_float(reuse[BR_QREF]);
+            double P = ((1.0 - (double)qr) / (double)qr) / ((1.0 - (double)q) / (double)q) * (1.0 + 1.0 / 65536.0);
+            for (int g = 0; g < G1; g++) { P *= (double)__uint_as_float(reuse[BR_RHO + g]); reuse[BR_RHO + g] = 0u; }
+            // a watch window costs about two windows of the full pass (one lookup per window instead of per pair, a list read,
+            // dependent loads): a list of more than a quarter of the windows does not pay, and is then rebuilt only every 8th full pass
+            const bool dense = eflags[0] != 0u, big = reuse[BR_WFULL] != 0u || 4ull * reuse[BR_WCOUNT] > nwin;
+            const bool watch = !dense && reuse[BR_VALID] != 0u && !big && P < (double)slack_pow;
+            const bool rebuild = !watch && !dense && !(big && ++reuse[BR_SKIP] % 8u != 0u);
+            reuse[BR_MODE] = watch ? 1u : rebuild ? 0u : 2u;
+            if (reuse[BR_VALID]) reuse[BR_LAMBDA] = __float_as_uint((float)log2(P));
+            if (watch) reuse[BR_WATCH]++;
+            else if (!dense) reuse[BR_FULL]++;
+            if (rebuild) {                                        // this full pass rebuilds the list (k_ebound clears VALID if it cannot)
+                reuse[BR_VALID] = 1u; reuse[BR_QREF] = __float_as_uint(q); reuse[BR_WCOUNT] = 0u; reuse[BR_WFULL] = 0u;
+            }
         }
     }
 }

@@ -177,6 +177,12 @@ int bamm_em_launch_count(bamm_em* em, uint64_t* kernels);
  * (always 1 when [0] is 0), [4] candidate windows listed by the bound pass of the last E-step, [5] windows in the active list,
  * [6] column passes of the exact plan, [7] the plain table rides in shared memory (0/1). */
 int bamm_em_estep_info(bamm_em* em, uint64_t info[8]);
+/* bound reuse of the pruned E-step (DESIGN.md §4.1; diagnostics, synchronises the EM stream): while the bound tables stay close
+ * to those of the last full bound pass, only the windows that pass listed within BAMM_BOUND_SLACK bits of the threshold are
+ * bounded again. info[0] reuse enabled for this object (0 with BAMM_NO_BOUND_REUSE), [1] full bound passes and [2] watch passes
+ * since creation, [3] windows in the watch list, [4] the last E-step took the watch pass (0/1), [5] the watch list is valid.
+ * *log2_drift: log2 of the last bound on how far the tables moved since the list was built (the watch pass needs < slack). */
+int bamm_em_bound_reuse_info(bamm_em* em, uint64_t info[6], float* log2_drift);
 void bamm_em_destroy(bamm_em* em);
 
 /* ---- multi-GPU (sequences sharded over ranks, one process per GPU; SURVEY.md §8e) ---------------------------- */
