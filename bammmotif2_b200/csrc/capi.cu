@@ -211,8 +211,9 @@ struct bamm_em {
     std::vector<uint32_t> dbg_tab_prev, dbg_tab_1, dbg_tab_3;
     unsigned long long* d_dbg_hist = nullptr;
     bool r_mat = true;          // d_r holds the posteriors of the last E-step (false after a pruned E-step until bamm_em_get_r)
-    const float *d_s_e = nullptr, *d_sT_e = nullptr, *d_tab_e = nullptr;   // the tables the last E-step read
+    const float *d_s_e = nullptr, *d_tab_e = nullptr;   // the tables the last E-step read
     float q_e = 0.3f;           // ... and its prior
+    float* d_s_keep = nullptr;  // copy of the s of the last E-step once a second update reuses its buffer (keep_last_estep)
     // active list (windows that survive the M-step's fixed-point rounding), one region per E-step warp
     uint32_t nregions = 0;
     ActiveEntry* d_act = nullptr;

@@ -129,8 +129,11 @@ struct CandList {
 // pass without the list (the last one was too long to pay); [BR_SKIP] full passes that kept a too long list; [BR_WFULL] a watch region filled up in the last list build; [BR_VALID] the watch list matches tab_ref and q_ref;
 // [BR_QREF] q of the full pass that built it (float bits); [BR_LAMBDA] log2 of the last drift bound (float bits);
 // [BR_FULL], [BR_WATCH] passes of each kind (diagnostics); [BR_WCOUNT] entries of the watch list;
-// [BR_RHO + g] max_e B_g[e] / tab_ref_g[e] of the tables built since the last E-step (float bits, k_make_bound_tables)
-constexpr int BR_MODE = 0, BR_VALID = 1, BR_QREF = 2, BR_LAMBDA = 3, BR_FULL = 4, BR_WATCH = 5, BR_WCOUNT = 6, BR_SKIP = 7, BR_WFULL = 8, BR_RHO = 9, BREUSE_WORDS = BR_RHO + MAXG;
+// [BR_PTAB] prod_g rho_g of the current tables against tab_ref, rounded up (float bits; k_estep_begin keeps it across E-steps that
+// follow no table build, 1 after a list build);
+// [BR_RHO + g] max_e B_g[e] / tab_ref_g[e] of the tables built since the last E-step (float bits, k_make_bound_tables; 0: none built)
+constexpr int BR_MODE = 0, BR_VALID = 1, BR_QREF = 2, BR_LAMBDA = 3, BR_FULL = 4, BR_WATCH = 5, BR_WCOUNT = 6, BR_SKIP = 7, BR_WFULL = 8, BR_PTAB = 9,
+              BR_RHO = 10, BREUSE_WORDS = BR_RHO + MAXG;
 // After an overflow the dense E-step runs for 2 iterations, then the bound pass tries again; every further overflow in a row
 // doubles the hold (a model whose posteriors stay diffuse pays log2(iterations) wasted bound passes, one that sharpens after
 // the first iterations is back on the pruned path at once); a pruned iteration that fits resets it.

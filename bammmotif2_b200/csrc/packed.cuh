@@ -273,6 +273,9 @@ __global__ void k_make_bound_tables(const float* __restrict__ s, const float* __
 // Rounding: b(p) and b_ref(p) are float products of G1 <= 8 factors, each within (1+2^-24)^7 of the exact product, thr within
 // a few ulps; the factor 1 + 2^-16 in P covers all of it. Intermediate products that end up subnormal lose relative accuracy,
 // but their absolute error (< 2^-149 times the remaining factors, each < 2^64) stays far below thr * 2^-m (> 2^-80 for m <= 32).
+// P has to bound the drift of the CURRENT tables, however many E-steps ran since they were built (estep, optimize_q, estep; the
+// E-steps of a dense hold): the table factor prod_g rho_g is kept in BR_PTAB and replaced only when tables were built since the
+// last E-step (some rho_g != 0; all of them 0 means every bound is 0, and any P is then right). The q ratio is formed afresh.
 __global__ void k_estep_begin(unsigned long long* __restrict__ scal, uint32_t* __restrict__ overflow, uint32_t* __restrict__ eflags,
                               uint32_t* __restrict__ reuse, float q, float slack_pow /* 2^m */, int G1, unsigned long long nwin) {
     if (threadIdx.x == 0) {
@@ -290,9 +293,13 @@ __global__ void k_estep_begin(unsigned long long* __restrict__ scal, uint32_t* _
             eflags[2] = 0u; eflags[3] = 0u;
         }
         if (reuse) {
+            bool built = false;
+            double T = 1.0;
+            for (int g = 0; g < G1; g++) { built |= reuse[BR_RHO + g] != 0u; T *= (double)__uint_as_float(reuse[BR_RHO + g]); reuse[BR_RHO + g] = 0u; }
+            if (built) reuse[BR_PTAB] = __float_as_uint(__double2float_ru(T));
             const float qr = __uint_as_float(reuse[BR_QREF]);
-            double P = ((1.0 - (double)qr) / (double)qr) / ((1.0 - (double)q) / (double)q) * (1.0 + 1.0 / 65536.0);
-            for (int g = 0; g < G1; g++) { P *= (double)__uint_as_float(reuse[BR_RHO + g]); reuse[BR_RHO + g] = 0u; }
+            const double P = ((1.0 - (double)qr) / (double)qr) / ((1.0 - (double)q) / (double)q) * (1.0 + 1.0 / 65536.0) *
+                             (double)__uint_as_float(reuse[BR_PTAB]);
             // a watch window costs about two windows of the full pass (one lookup per window instead of per pair, a list read,
             // dependent loads): a list of more than a quarter of the windows does not pay, and is then rebuilt only every 8th full pass
             const bool dense = eflags[0] != 0u, big = reuse[BR_WFULL] != 0u || 4ull * reuse[BR_WCOUNT] > nwin;
@@ -304,6 +311,7 @@ __global__ void k_estep_begin(unsigned long long* __restrict__ scal, uint32_t* _
             else if (!dense) reuse[BR_FULL]++;
             if (rebuild) {                                        // this full pass rebuilds the list (k_ebound clears VALID if it cannot)
                 reuse[BR_VALID] = 1u; reuse[BR_QREF] = __float_as_uint(q); reuse[BR_WCOUNT] = 0u; reuse[BR_WFULL] = 0u;
+                reuse[BR_PTAB] = __float_as_uint(1.0f);           // tab_ref becomes the current tables
             }
         }
     }
