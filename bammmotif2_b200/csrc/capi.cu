@@ -180,7 +180,6 @@ struct bamm_em {
     uint32_t* d_pk_ids = nullptr;   uint64_t* d_pk_roff = nullptr;
     Plan plan;                  // W, K, Yn for the packed M-step / scoring kernels
     std::vector<GroupPlan> gplans;   // column groups of the packed E-step, one plan per column pass (chosen in set_model)
-    std::vector<char> gfast;         // per pass: every group's bit field sits below bit 32 of the window word
     size_t tab_capacity = 0;    // bytes available for the group tables (= opt-in shared memory)
     float* d_tab = nullptr;     // group tables, concatenated; tab_capacity bytes per pass
     float* d_tab_alt = nullptr; // second buffer: launch_update writes the next tables there and swaps, so the tables of the last
@@ -191,7 +190,7 @@ struct bamm_em {
     bool cand_ok = false;       // candidate list allocated (bamm_em_create)
     bool sparse = false;        // the current plans use the pruned path (bamm_em_set_model)
     bool stage = false;         // the exact pass stages the sequence words in shared memory
-    GroupPlan bplan; bool bfast = false;
+    GroupPlan bplan;
     BoundLevels blev;
     float* d_btab = nullptr;    // bound tables
     float* d_U = nullptr;       // maxima of s over dropped context bases, per level
@@ -206,10 +205,6 @@ struct bamm_em {
     uint32_t* d_watch = nullptr; uint64_t* d_wreg_off = nullptr; uint2* d_watch_seq = nullptr;
     float* d_btab_ref = nullptr; uint32_t* d_reuse = nullptr;
     int bound_slack = 10;           // m: the watch list holds the windows whose bound reaches thr 2^-m (BAMM_BOUND_SLACK)
-    // BAMM_DEBUG_BOUND (capi_em.inl, debug_bound): pruned E-steps since set_model, bound tables of the previous / first / third one
-    int dbg_estep = 0;
-    std::vector<uint32_t> dbg_tab_prev, dbg_tab_1, dbg_tab_3;
-    unsigned long long* d_dbg_hist = nullptr;
     bool r_mat = true;          // d_r holds the posteriors of the last E-step (false after a pruned E-step until bamm_em_get_r)
     const float *d_s_e = nullptr, *d_tab_e = nullptr;   // the tables the last E-step read
     float q_e = 0.3f;           // ... and its prior
@@ -236,13 +231,10 @@ struct bamm_em {
     uint64_t* d_reg_off = nullptr;
     uint16_t* d_ypatch = nullptr;   // owned by the seqset
     int grid_pe = 0, block_pe = 1024;
-    size_t smem_pe = 0;
     uint32_t nparts = 1;
     uint32_t gen_nrep = 1;          // generic M-step without shared-memory tables: copies of the global count table
     int gen_nsplit = 0, gen_nc = 0; // ... or column ranges with shared-memory low words (k_mstep_cols), 0 = off
     // device
-    uint32_t* d_seq_ids = nullptr;
-    uint64_t* d_r_off = nullptr;
     float* d_r = nullptr;
     float* d_s = nullptr;         // [j][y]
     float* d_sT = nullptr;        // the same table in the reference's [y][j] order (row gathers of the patched k-mers)
@@ -268,8 +260,7 @@ struct bamm_em {
     std::vector<uint64_t> h_r_off;
     float q = 0.3f;
     float llh = 0.0f;
-    bool model_set = false, s_valid = false, r_valid = false;
-    float t_e = 0, t_m = 0;
+    bool model_set = false, r_valid = false;
 };
 
 // ------------------------------------------------------------------------------------------- library / device

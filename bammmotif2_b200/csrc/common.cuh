@@ -62,6 +62,9 @@ struct GroupPlan {
     int pass_first, pass_last;
     float thr0;                  // 2^-41 (1-q) 0.999: smallest unnormalised value that can reach the M-step's threshold (norm >= 1-q)
 };
+// every group's bit field sits below bit 32 of the window word, so one shift extracts it (the kernels' FAST variant). Group 0
+// ends at the lowest column and has the largest shift; the planners place it at <= 30 when they can and at >= 32 otherwise.
+inline bool one_shift(const GroupPlan& gp) { return gp.shift[0] < 32; }
 
 // ---- window extraction ---------------------------------------------------------------------------------------------
 // 64 bits holding bases b0 .. b0+31 of a sequence (b0 >= -32: the pad words supply leading zeros), as (hi, lo).

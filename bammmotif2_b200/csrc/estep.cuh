@@ -538,58 +538,6 @@ k_ebound_watch(PackedView pv, const __grid_constant__ GroupPlan gp, const float*
     if (lane == 0 && cpos) atomicAdd(reinterpret_cast<unsigned long long*>(cl.flags + 2), (unsigned long long)cpos);
 }
 
-// ---- diagnostic (BAMM_DEBUG_BOUND): distribution of the bounds relative to the candidate threshold ---------------------
-// Same windows, tables and products as k_ebound; instead of a list, a histogram of log2(b(p) / thr) in quarter bits
-// (bin BOUND_HIST_ZERO + floor(4 log2), clamped; bin 0 also takes b = 0). One shared-memory histogram per CTA, one flush.
-constexpr int BOUND_HIST_BINS = 512, BOUND_HIST_ZERO = 384;
-template <int G1, bool FAST>
-__global__ void __launch_bounds__(BAMM_E_THREADS, 1)
-k_ebound_hist(PackedView pv, const __grid_constant__ GroupPlan gp, const float* __restrict__ tab_g, unsigned long long* __restrict__ hist) {
-    extern __shared__ __align__(16) float tab[];
-    __shared__ unsigned long long stage_bar;
-    __shared__ uint32_t h[BOUND_HIST_BINS];
-    for (int i = threadIdx.x; i < BOUND_HIST_BINS; i += blockDim.x) h[i] = 0u;
-    bulk_stage_begin(tab, tab_g, gp.table_bytes, &stage_bar);
-    bulk_stage_wait(&stage_bar);
-    __syncthreads();
-    const int lane = threadIdx.x & 31;
-    const uint32_t warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    const uint32_t nwarps = gridDim.x * (blockDim.x >> 5);
-    const int W = gp.W, K = gp.K, KD = gp.kd;
-    const uint32_t tab_s = (uint32_t)__cvta_generic_to_shared(tab);
-    GroupConsts<G1> gc; load_consts<G1>(gc, gp, tab_s);
-    auto bin_of = [](float b, float thr) {
-        if (!(b > 0.0f)) return 0;
-        const int k = (int)floorf(4.0f * log2f(b / thr)) + BOUND_HIST_ZERO;
-        return min(max(k, 0), BOUND_HIST_BINS - 1);
-    };
-    for (uint32_t li = warp; li < pv.nlist; li += nwarps) {
-        const PackedSeq sq = pv.seqs[pv.seq_ids[li]];
-        const int L = (int)sq.L, LW1 = L - W + 1, mid = (int)sq.mid;
-        const float thr = gp.thr0 * (float)LW1 / gp.q;
-        const int tl = min(max(L - 2 * W + 2, 0), LW1);
-        int n0 = tl, n1 = tl;
-        if (mid >= 0) { n0 = min(max(mid - W + 1, 0), tl); n1 = min(mid + K + 1, tl); }
-        const uint32_t* __restrict__ wseq = pv.words + sq.word_off;
-        for (int c = 0; c < (tl + 63) >> 6; c++) {
-            const int p = 64 * c + 2 * lane;
-            uint32_t whi, wlo;
-            window_bits(wseq, p - KD, whi, wlo);
-            float b0 = 1.0f, b1 = 1.0f;
-#pragma unroll
-            for (int g = 0; g < G1; g++) {
-                const uint32_t e = __float_as_uint(lds_f32(group_offset<G1, FAST>(gc, g, whi, wlo), gc.ab[g]));
-                const float f0 = __uint_as_float(e << 16), f1 = __uint_as_float(e & 0xffff0000u);
-                b0 = g ? b0 * f0 : f0; b1 = g ? b1 * f1 : f1;
-            }
-            if (p < tl && (p < n0 || p >= n1)) atomicAdd(&h[bin_of(b0, thr)], 1u);
-            if (p + 1 < tl && (p + 1 < n0 || p + 1 >= n1)) atomicAdd(&h[bin_of(b1, thr)], 1u);
-        }
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < BOUND_HIST_BINS; i += blockDim.x) if (h[i]) atomicAdd(&hist[i], (unsigned long long)h[i]);
-}
-
 // ---- pruned E-step, part 0: the windows over the N and the truncated tail ----------------------------------------------
 // Every sequence has W+K windows over the structural N and W-1 truncated windows (EM.cpp:167); they need the masked evaluation
 // and most truncated ones are active, so they are evaluated for all sequences — with the sequences ACROSS the lanes: lane l

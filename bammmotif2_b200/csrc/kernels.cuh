@@ -113,17 +113,14 @@ struct SubsetView {
 // from the reference only through the summation order inside norm. One warp per sequence; lanes = window starts.
 // Scalars (log likelihood, sum of r for optimize_q) are accumulated per warp as 2^32 fixed point and added to
 // the exchange buffer with one 64-bit atomic per warp: integer sums => order-independent result.
-template <typename YT, bool SMEM>
+template <typename YT>
 __global__ void __launch_bounds__(512)
-k_estep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float* __restrict__ s_g /* SMEM: [j][y]; else [y][j] */, float q,
+k_estep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float* __restrict__ s_g /* [j][y] */, float q,
         float* __restrict__ r, unsigned long long* __restrict__ scal /* [0]=llh_fx, [1]=rsum_fx */) {
     extern __shared__ float s_sh[];
-    const float* s = s_g;
-    if (SMEM) {
-        for (uint32_t i = threadIdx.x; i < (uint32_t)W * Yn; i += blockDim.x) s_sh[i] = s_g[i];
-        __syncthreads();
-        s = s_sh;
-    }
+    for (uint32_t i = threadIdx.x; i < (uint32_t)W * Yn; i += blockDim.x) s_sh[i] = s_g[i];
+    __syncthreads();
+    const float* s = s_sh;
     const int lane = threadIdx.x & 31;
     const uint32_t warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const uint32_t nwarps = gridDim.x * (blockDim.x >> 5);
@@ -158,9 +155,7 @@ k_estep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float
             float prod = 1.0f;
             for (int j = 0; j < W; j++) {
                 const uint32_t y = st.get(lane, j);
-                // table in global memory: the [y][j] copy, where the entries lane p reads at column j and lane p+1 read at
-                // column j-1 share a row (same k-mer) => neighbouring lanes reuse the line in L1 one step later
-                if (j <= jmax) prod *= SMEM ? s[(uint32_t)j * Yn + y] : __ldg(s + (y * (uint32_t)W + (uint32_t)j));
+                if (j <= jmax) prod *= s[(uint32_t)j * Yn + y];
             }
             if (p < LW1) {
                 const float val = prod * pos;
@@ -188,8 +183,8 @@ k_estep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float
 // E-step for tables beyond shared memory, row form. The lanes of a warp own 32 consecutive POSITIONS: lane l loads the whole
 // table row of its k-mer, s[y(i)][0..W) — W4/4 16-byte loads from the padded [y][W4] copy of the table — and window p takes
 // column j from the lane that owns position p+j with one shuffle. A warp then touches 32 rows per 32 windows (3 load
-// instructions at W = 12) where k_estep<., false> issues W gathers of 32 scattered addresses each: the L1 wavefronts, which
-// bound that kernel (ncu: 92 % of the LSU wavefront peak), drop by W / (W4/4). Same factors multiplied in the same order =>
+// instructions at W = 12) where gathering one column at a time from the [y][j] table in global memory issues W gathers of 32
+// scattered addresses each: the L1 wavefronts, which bound that form (ncu: 92 % of the LSU wavefront peak), drop by W / (W4/4). Same factors multiplied in the same order =>
 // the same r, bit for bit. The rows of the next 32 positions and the k-mer indices of the 32 after them are in flight while
 // the current round is multiplied.
 __global__ void k_pad_rows(const float* __restrict__ sT /* [y][W] */, int W, int W4, uint32_t Yn, float* __restrict__ out /* [y][W4] */) {

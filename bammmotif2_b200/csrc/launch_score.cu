@@ -12,8 +12,9 @@ static int score_zoops_one(const GroupPlan& gp, int sms, cudaStream_t st, const 
     k_score_zoops_packed<G, FAST><<<sms, 1024, smem, st>>>(pv, gp, d_tab, d_s, two_eps, d_zoops, d_z, d_out);
     return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
-int launch_score_zoops(const GroupPlan& gp, bool fast, int sms, cudaStream_t st, const PackedView& pv, const float* d_tab, const float* d_s,
+int launch_score_zoops(const GroupPlan& gp, int sms, cudaStream_t st, const PackedView& pv, const float* d_tab, const float* d_s,
                        float two_eps, float* d_zoops, unsigned long long* d_z, const uint32_t* d_out, size_t plain_bytes) {
+    const bool fast = one_shift(gp);
     switch (gp.G) {
 #define X(g) case g: return fast ? score_zoops_one<g, true>(gp, sms, st, pv, d_tab, d_s, two_eps, d_zoops, d_z, d_out, plain_bytes) \
                                  : score_zoops_one<g, false>(gp, sms, st, pv, d_tab, d_s, two_eps, d_zoops, d_z, d_out, plain_bytes);
