@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "../../include/bamm_b200.h"       // BAMM_MAX_MOTIF_WIDTH sizes per-column arrays in the kernels
 
 namespace bamm {
 

@@ -72,7 +72,7 @@ __global__ void k_count_kmers(const YT* __restrict__ Y, uint64_t npos, uint32_t 
 
 // ---------------------------------------------------------------------------------------------------------
 // Sliding k-mer window of a warp: lane l holds y[p0+l] and y[p0+32+l]; the k-mer under motif column j of the
-// window that starts at p0+l is element l+j of that 64-entry strip (W <= 32), fetched with one shuffle.
+// window that starts at p0+l is element l+j of that 64-entry strip (W <= 32; wider motifs: BlockStrip), fetched with one shuffle.
 template <typename YT> struct Strip;
 template <> struct Strip<uint16_t> {
     uint32_t packed;
@@ -98,6 +98,50 @@ template <> struct Strip<uint32_t> {
     }
 };
 
+// Column blocks of a wide motif (DESIGN.md §4.6): columns [32b, min(W, 32b+32)) for b < NB form block b, and the strip holds
+// NB+1 segments of 32 k-mer indices, seg[s] = y[p0 + 32s + lane]. Block b reads the pair (seg[b], seg[b+1]) with the shuffle of
+// Strip::get, so j still ascends from 0 and every product and sum keeps its order. NB = 1 is the Strip above (W <= 32).
+template <typename YT, int NB> struct BlockStrip {
+    uint32_t seg[NB + 1];
+    __device__ __forceinline__ void load(const YT* __restrict__ y, uint64_t p, uint64_t L) {
+#pragma unroll
+        for (int s = 0; s <= NB; s++) seg[s] = (p + 32 * s < L) ? (uint32_t)y[p + 32 * s] : 0u;
+    }
+    // the strip of the windows 32 further on: the segments shift by one, one new segment is loaded
+    __device__ __forceinline__ void load_next(const BlockStrip& cur, const YT* __restrict__ y, uint64_t p /* first new window */, uint64_t L) {
+#pragma unroll
+        for (int s = 0; s < NB; s++) seg[s] = cur.seg[s + 1];
+        seg[NB] = (p + 32 * NB < L) ? (uint32_t)y[p + 32 * NB] : 0u;
+    }
+    __device__ __forceinline__ uint32_t get(int lane, int b, int jj) const {
+        const int src = lane + jj;
+        const uint32_t ta = __shfl_sync(FULL, seg[b], src & 31), tb = __shfl_sync(FULL, seg[b + 1], src & 31);
+        return (src < 32) ? ta : tb;
+    }
+};
+template <typename YT> struct BlockStrip<YT, 1> {
+    Strip<YT> st;
+    __device__ __forceinline__ void load(const YT* __restrict__ y, uint64_t p, uint64_t L) { st.load(y, p, L); }
+    __device__ __forceinline__ void load_next(const BlockStrip&, const YT* __restrict__ y, uint64_t p, uint64_t L) { st.load(y, p, L); }
+    __device__ __forceinline__ uint32_t get(int lane, int, int jj) const { return st.get(lane, jj); }
+};
+// f(b, jj) for the columns j = 32 b + jj, j = 0 .. W-1 in ascending order
+template <int NB, typename F>
+__device__ __forceinline__ void for_columns(int W, F&& f) {
+    if (NB == 1) {
+        for (int j = 0; j < W; j++) f(0, j);
+    } else {
+#pragma unroll
+        for (int b = 0; b < NB; b++) {
+            const int nc = min(W - 32 * b, 32);
+#pragma unroll 8                                // the default unrolling spills in k_score
+            for (int jj = 0; jj < nc; jj++) f(b, jj);
+        }
+    }
+}
+// column blocks a width needs (1 for W <= 32, 2 up to BAMM_MAX_MOTIF_WIDTH)
+static inline int column_blocks(int W) { return W > 32 ? 2 : 1; }
+
 struct SubsetView {
     const uint64_t* seq_off;   // seqset offsets (nseq+1)
     const uint32_t* seq_ids;   // subset -> seqset index, or nullptr for identity
@@ -113,7 +157,8 @@ struct SubsetView {
 // from the reference only through the summation order inside norm. One warp per sequence; lanes = window starts.
 // Scalars (log likelihood, sum of r for optimize_q) are accumulated per warp as 2^32 fixed point and added to
 // the exchange buffer with one 64-bit atomic per warp: integer sums => order-independent result.
-template <typename YT>
+// NB: column blocks (column_blocks(W)).
+template <typename YT, int NB>
 __global__ void __launch_bounds__(512)
 k_estep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float* __restrict__ s_g /* [j][y] */, float q,
         float* __restrict__ r, unsigned long long* __restrict__ scal /* [0]=llh_fx, [1]=rsum_fx */) {
@@ -147,16 +192,17 @@ k_estep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float
         hd = hn;
         const float pos = q / (float)LW1;
         float sum = 0.0f;
-        Strip<YT> st; st.load(yn, lane, L);
+        BlockStrip<YT, NB> st; st.load(yn, lane, L);
         for (uint64_t p0 = 0; p0 < LW1; p0 += 32) {
             const uint64_t p = p0 + lane;
-            Strip<YT> nx; nx.load(yn, p + 32, L);
+            BlockStrip<YT, NB> nx; nx.load_next(st, yn, p + 32, L);
             const int jmax = (p < LW1) ? (int)min((uint64_t)(W - 1), L - W - p) : -1;
             float prod = 1.0f;
-            for (int j = 0; j < W; j++) {
-                const uint32_t y = st.get(lane, j);
+            for_columns<NB>(W, [&](int b, int jj) {
+                const int j = 32 * b + jj;
+                const uint32_t y = st.get(lane, b, jj);
                 if (j <= jmax) prod *= s[(uint32_t)j * Yn + y];
-            }
+            });
             if (p < LW1) {
                 const float val = prod * pos;
                 rn[L - W - p] = val;
@@ -187,6 +233,10 @@ k_estep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float
 // scattered addresses each: the L1 wavefronts, which bound that form (ncu: 92 % of the LSU wavefront peak), drop by W / (W4/4). Same factors multiplied in the same order =>
 // the same r, bit for bit. The rows of the next 32 positions and the k-mer indices of the 32 after them are in flight while
 // the current round is multiplied.
+// A motif wider than 32 columns takes two column passes, PASS 1 over columns [0, 32) and PASS 2 over [32, W), and the product of
+// PASS 1 is stored in r: the rows of both blocks for this round and the next would be 4 x 32 floats per lane, beyond the 128
+// registers of a 512-thread CTA. PASS 2 continues the product from the stored float, so the factors are multiplied in the same
+// order. PASS 0 takes all W <= 32 columns at once. RS: row stride of the padded table in PASS 1 / 2 (PASS 0: W4).
 __global__ void k_pad_rows(const float* __restrict__ sT /* [y][W] */, int W, int W4, uint32_t Yn, float* __restrict__ out /* [y][W4] */) {
     const uint32_t total = Yn * (uint32_t)W4;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
@@ -194,15 +244,18 @@ __global__ void k_pad_rows(const float* __restrict__ sT /* [y][W] */, int W, int
         out[i] = j < (uint32_t)W ? sT[y * (uint32_t)W + j] : 1.0f;
     }
 }
-template <typename YT, int W4>
-__global__ void __launch_bounds__(512)
-k_estep_rows(const YT* __restrict__ Y, SubsetView sv, int W, const float* __restrict__ rows /* [y][W4] */, float q,
+// PASS 1 / 2 ask ptxas for one CTA per SM: its occupancy heuristic otherwise caps the PASS 2 instantiations near 64 registers and spills
+template <typename YT, int W4, int PASS>
+__global__ void __launch_bounds__(512, PASS == 0 ? 0 : 1)
+k_estep_rows(const YT* __restrict__ Y, SubsetView sv, int W, const float* __restrict__ rows /* [y][RS] */, int RS, float q,
              float* __restrict__ r, unsigned long long* __restrict__ scal /* [0]=llh_fx, [1]=rsum_fx */) {
+    constexpr int C0 = PASS == 2 ? 32 : 0;                                      // first column of this pass
     const int lane = threadIdx.x & 31;
     const uint32_t warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const uint32_t nwarps = gridDim.x * (blockDim.x >> 5);
     long long llh_fx = 0, rsum_fx = 0;
     const float one_minus_q = 1.0f - q;
+    const int nc = PASS == 1 ? 32 : W - C0;                                     // columns of this pass
     struct Hdr { uint64_t base, L, roff; };
     auto load_hdr = [&](uint64_t i) {
         Hdr h; h.base = 0; h.L = 0; h.roff = 0;
@@ -213,7 +266,7 @@ k_estep_rows(const YT* __restrict__ Y, SubsetView sv, int W, const float* __rest
         return h;
     };
     auto load_row = [&](float (&dst)[W4], bool on, uint32_t y) {
-        const float4* __restrict__ src = reinterpret_cast<const float4*>(rows + (size_t)y * W4);
+        const float4* __restrict__ src = reinterpret_cast<const float4*>(rows + (size_t)y * (PASS == 0 ? W4 : RS) + C0);
 #pragma unroll
         for (int qd = 0; qd < W4 / 4; qd++) {
             float4 v = make_float4(1.0f, 1.0f, 1.0f, 1.0f);
@@ -231,29 +284,34 @@ k_estep_rows(const YT* __restrict__ Y, SubsetView sv, int W, const float* __rest
         const float pos = q / (float)LW1;
         float sum = 0.0f;
         float cur[W4], nxt[W4];
-        load_row(cur, (uint32_t)lane < L, (uint32_t)lane < L ? (uint32_t)yn[lane] : 0u);
-        uint32_t y1 = 32u + lane < L ? (uint32_t)yn[32 + lane] : 0u;           // k-mer of this lane's position in the next round
+        load_row(cur, (uint32_t)lane + C0 < L, (uint32_t)lane + C0 < L ? (uint32_t)yn[lane + C0] : 0u);
+        uint32_t y1 = 32u + C0 + lane < L ? (uint32_t)yn[32 + C0 + lane] : 0u;   // k-mer of this lane's position in the next round
         for (uint32_t p0 = 0; p0 < LW1; p0 += 32) {
             const uint32_t p = p0 + lane;
-            load_row(nxt, p + 32 < L, y1);
-            y1 = p + 64 < L ? (uint32_t)yn[p + 64] : 0u;
-            const int jmax = (p < LW1) ? (int)min((uint32_t)(W - 1), L - W - p) : -1;
-            float prod = 1.0f;
+            load_row(nxt, p + C0 + 32 < L, y1);
+            y1 = p + C0 + 64 < L ? (uint32_t)yn[p + C0 + 64] : 0u;
+            const int jmax = (p < LW1) ? (int)min((uint32_t)(W - 1), L - W - p) - C0 : -1;    // last column of this pass
+            float prod = (PASS == 2 && p < LW1) ? rn[L - W - p] : 1.0f;
 #pragma unroll
             for (int j = 0; j < W4; j++) {
-                // position p+j belongs to lane (lane+j) mod 32 of this round if lane+j < 32, of the next round otherwise
-                if (j >= W) break;                                                   // padding columns (uniform)
+                // position p+C0+j belongs to lane (lane+j) mod 32 of this round if lane+j < 32, of the next round otherwise
+                if (j >= nc) break;                                                  // padding columns (uniform)
                 const float v = __shfl_sync(FULL, lane >= j ? cur[j] : nxt[j], (lane + j) & 31);
                 if (j <= jmax) prod *= v;
             }
             if (p < LW1) {
-                const float val = prod * pos;
-                rn[L - W - p] = val;
-                sum += val;
+                if (PASS == 1) {
+                    rn[L - W - p] = prod;
+                } else {
+                    const float val = prod * pos;
+                    rn[L - W - p] = val;
+                    sum += val;
+                }
             }
 #pragma unroll
             for (int j = 0; j < W4; j++) cur[j] = nxt[j];
         }
+        if (PASS == 1) continue;
         sum = warp_sum(sum);
         const float norm = one_minus_q + sum;
         __syncwarp();
@@ -276,7 +334,7 @@ k_estep_rows(const YT* __restrict__ Y, SubsetView sv, int W, const float* __rest
 // atomics to the low word of a CTA-private table; the returned old value tells whether the low word wrapped,
 // and the carry (plus the high word of large r) goes to the CTA's 64-bit partial table in global memory.
 // No floating-point atomics anywhere => the sum is exact in fixed point and independent of execution order.
-template <typename YT, bool SMEM>
+template <typename YT, bool SMEM, int NB /* column blocks, as k_estep */>
 __global__ void __launch_bounds__(512)
 k_mstep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float* __restrict__ r,
         unsigned long long* __restrict__ part /* SMEM: [gridDim.x][W*Yn]; else nrep [W*Yn] tables shared by the CTAs */, uint32_t nrep) {
@@ -300,7 +358,7 @@ k_mstep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float
         const float* __restrict__ rn = r + sv.r_off[i];
         for (uint64_t p0 = 0; p0 < LW1; p0 += 32) {
             const uint64_t p = p0 + lane;
-            Strip<YT> st; st.load(yn, p, L);
+            BlockStrip<YT, NB> st; st.load(yn, p, L);
             int jmax = -1;
             unsigned long long X = 0;
             if (p < LW1) {
@@ -309,8 +367,9 @@ k_mstep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float
                 if (X == 0) jmax = -1;
             }
             const uint32_t xlo = (uint32_t)X, xhi = (uint32_t)(X >> 32);
-            for (int j = 0; j < W; j++) {
-                const uint32_t y = st.get(lane, j);
+            for_columns<NB>(W, [&](int b, int jj) {
+                const int j = 32 * b + jj;
+                const uint32_t y = st.get(lane, b, jj);
                 if (j <= jmax) {
                     const uint32_t bin = (uint32_t)j * Yn + y;
                     if (SMEM) {
@@ -321,7 +380,7 @@ k_mstep(const YT* __restrict__ Y, SubsetView sv, int W, uint32_t Yn, const float
                         atomicAdd(&mypart[bin], X);
                     }
                 }
-            }
+            });
         }
     }
     if (SMEM) {
@@ -574,6 +633,7 @@ __device__ __forceinline__ void update_model_body(ModelDims d, const unsigned lo
     const uint32_t crank = CL == 1 ? 0u : cooperative_groups::this_cluster().block_rank();
     const uint32_t tid = crank * blockDim.x + threadIdx.x, nt = CL * blockDim.x;
     __shared__ float sumN[64];
+    static_assert(BAMM_MAX_MOTIF_WIDTH <= 64, "sumN holds one sum per column");
     __shared__ double red[32];
     // top-order counts: fixed point -> float, [j][y] -> [y][j]
     float* nK = n_all + d.voff[K];
@@ -692,7 +752,7 @@ __global__ void k_make_s(ModelDims d, const float* __restrict__ v_all, const flo
 // Scoring. reference: ScoreSeqSet::calcLogOdds, src/seq_scoring/ScoreSeqSet.cpp:25-67. Full windows (all W
 // columns, :49-54), float sum in ascending j from 0.0f (bit-identical to the reference for the same table),
 // per-sequence maximum with the FIRST maximal window winning (strict '>' scan, :59-62).
-template <typename YT, bool SMEM>
+template <typename YT, bool SMEM, int NB /* column blocks, as k_estep */>
 __global__ void __launch_bounds__(512)
 k_score(const YT* __restrict__ Y, SubsetView sv, const uint64_t* __restrict__ mops_off, int W, uint32_t Yn,
         const float* __restrict__ s_g, float* __restrict__ zoops, unsigned long long* __restrict__ z,
@@ -717,12 +777,12 @@ k_score(const YT* __restrict__ Y, SubsetView sv, const uint64_t* __restrict__ mo
         uint64_t bestp = 0;
         for (uint64_t p0 = 0; p0 < LW1; p0 += 32) {
             const uint64_t p = p0 + lane;
-            Strip<YT> st; st.load(yn, p, L);
+            BlockStrip<YT, NB> st; st.load(yn, p, L);
             float sc = 0.0f;
-            for (int j = 0; j < W; j++) {
-                const uint32_t y = st.get(lane, j);
-                sc += s[(uint32_t)j * Yn + y];
-            }
+            for_columns<NB>(W, [&](int b, int jj) {
+                const uint32_t y = st.get(lane, b, jj);
+                sc += s[(uint32_t)(32 * b + jj) * Yn + y];
+            });
             if (p < LW1) {
                 if (mops) mops[mops_off[oi] + p] = sc;
                 if (sc > best) { best = sc; bestp = p; }

@@ -24,7 +24,7 @@ struct MaskView {
 template <typename YT>
 __global__ void __launch_bounds__(256)
 k_mask_phase1(const YT* __restrict__ Y, MaskView mv, int W, uint32_t A, const float* __restrict__ s0_g, float q, float* __restrict__ r) {
-    __shared__ float s0[6 * 32];
+    __shared__ float s0[6 * BAMM_MAX_MOTIF_WIDTH];
     for (uint32_t i = threadIdx.x; i < A * (uint32_t)W; i += blockDim.x) s0[i] = s0_g[i];
     __syncthreads();
     const int lane = threadIdx.x & 31;
@@ -192,7 +192,7 @@ k_pwm_sample_sites(const YT* __restrict__ Y, const uint64_t* __restrict__ seq_of
                    int W, int K, uint32_t A, uint32_t asize, const float* __restrict__ score_g /* [asize][W] */, float q,
                    const double* __restrict__ uniforms, float* __restrict__ scratch, uint64_t scratch_stride,
                    int* __restrict__ n_all, const uint32_t* __restrict__ voff /* [K+2] */, unsigned long long* __restrict__ z_out) {
-    __shared__ float score[6 * 32];
+    __shared__ float score[6 * BAMM_MAX_MOTIF_WIDTH];
     for (uint32_t i = threadIdx.x; i < asize * (uint32_t)W; i += blockDim.x) score[i] = score_g[i];
     __syncthreads();
     const int lane = threadIdx.x & 31;

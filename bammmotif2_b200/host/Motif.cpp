@@ -42,7 +42,7 @@ void Motif::bindViews(){
 Motif::Motif( size_t length, size_t K, std::vector<float> alpha, float** v_bg, size_t k_bg, float glob_q )
     : W_( length ), K_( K ), q_( glob_q ), v_bg_( v_bg ), k_bg_( k_bg ){
     if( W_ < 1 || W_ > BAMM_MAX_MOTIF_WIDTH ){
-        // the device kernels keep one window (W columns + K context bases) in a 32-base word; the reference has no such limit
+        // the device path takes motifs of up to BAMM_MAX_MOTIF_WIDTH columns (include/bamm_b200.h); the reference has no such limit
         std::cerr << "Error: motif width " << W_ << " (including --extend columns) is outside [1, " << BAMM_MAX_MOTIF_WIDTH
                   << "], the range of the B200 path." << std::endl;
         exit( 1 );
