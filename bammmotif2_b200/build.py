@@ -2,6 +2,7 @@
 
     libbamm_b200.so   the C-ABI library (include/bamm_b200.h): csrc/capi.cu (+ capi_*.inl, one translation unit) + csrc/*.cuh, sm_100a only
     bin/BaMMmotif     the C++ host side (host/*.cpp: the reference's class surface over the C ABI) as the drop-in CLI
+    bin/BaMMScan      the occurrence scan over the same host classes (host/mainScan.cpp)
     bin/host_check    test helper for the CPU-only parts of the host classes
 
 Run as `python -m bammmotif2_b200.build` or through __graft_entry__.build().
@@ -79,7 +80,7 @@ HOST_FLAGS = ["-std=c++17", "-O2", "-Wall", "-ffp-contract=off", "-pthread"]
 
 
 def build_host(force=False):
-    """host/*.cpp -> bin/BaMMmotif and bin/host_check, linked against libbamm_b200.so (rpath $ORIGIN/..)."""
+    """host/*.cpp -> bin/BaMMmotif, bin/BaMMScan and bin/host_check, linked against libbamm_b200.so (rpath $ORIGIN/..)."""
     hdir, bdir, odir = os.path.join(HERE, "host"), os.path.join(HERE, "bin"), os.path.join(HERE, "build", "host")
     os.makedirs(bdir, exist_ok=True)
     os.makedirs(odir, exist_ok=True)
@@ -87,13 +88,13 @@ def build_host(force=False):
     env = {k: v for k, v in os.environ.items() if k not in ("CC", "CXX")}
     headers = [os.path.join(hdir, f) for f in os.listdir(hdir) if f.endswith(".h")] + [os.path.join(ROOT, "include", "bamm_b200.h"), __file__]
     objs = {}
-    for name in HOST_SOURCES + ["mainBaMM", "host_check"]:
+    for name in HOST_SOURCES + ["mainBaMM", "mainScan", "host_check"]:
         src, obj = os.path.join(hdir, name + ".cpp"), os.path.join(odir, name + ".o")
         if force or not _newer(obj, [src] + headers):
             subprocess.check_call([gxx] + HOST_FLAGS + ["-c", src, "-o", obj], env=env)
         objs[name] = obj
     outs = []
-    for exe, main in (("BaMMmotif", "mainBaMM"), ("host_check", "host_check")):
+    for exe, main in (("BaMMmotif", "mainBaMM"), ("BaMMScan", "mainScan"), ("host_check", "host_check")):
         out = os.path.join(bdir, exe)
         deps = [objs[n] for n in HOST_SOURCES] + [objs[main]]
         if force or not _newer(out, deps + [LIB]):

@@ -78,7 +78,15 @@ SIGNATURES = {
     "bamm_sort_scores": (C.c_int, [_f32p, C.c_uint64, C.c_int]),
     "bamm_mops_pvalues": (C.c_int, [_f32p, C.c_uint64, _f32p, C.c_uint64, C.c_uint64, _f32p, _f32p]),
     "bamm_score_logodds": (C.c_int, [_vp, _u64p, C.c_uint64, C.c_int, C.c_int, C.c_int, _f32p, _f32p, _f32p, _u64p, _f32p]),
+    "bamm_scan_create": (C.c_int, [_vp, _u64p, C.c_uint64, C.c_int, C.c_int, C.c_int, _f32p, _f32p, C.POINTER(_vp)]),
+    "bamm_scan_hits": (C.c_int, [_vp, _vp, _u64p, C.c_uint64, C.c_uint64, C.c_float, _u64p, _vp, C.c_uint64, _u64p]),
+    "bamm_scan_info": (C.c_int, [_vp, _u64p, _f32p, _f32p, _f32p]),
+    "bamm_scan_destroy": (None, [_vp]),
 }
+
+# struct bamm_hit of include/bamm_b200.h
+HIT_DTYPE = np.dtype([("seq", np.uint64), ("window", np.uint64), ("score", np.float32), ("p_value", np.float32),
+                      ("e_value", np.float32), ("reserved", np.uint32)])
 
 _lib = None
 
@@ -479,6 +487,58 @@ class EM:
     def close(self):
         if self.h:
             load().bamm_em_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class Scan:
+    """Occurrence scan of one motif (bamm_scan): the negative windows of `negset[subset]` are scored and sorted on the device
+    once; hits() then returns the windows of a positive set whose p-value is < p_cutoff."""
+
+    def __init__(self, negset, W, K, K_bg_model, v_all, vbg_all, subset=None):
+        sub = np.ascontiguousarray(subset, np.uint64) if subset is not None else None
+        v = np.ascontiguousarray(v_all, np.float32)
+        vb = np.ascontiguousarray(vbg_all, np.float32)
+        h = _vp()
+        _check(load().bamm_scan_create(negset.h if negset is not None else None, _ptr(sub, _u64p), len(sub) if sub is not None else 0,
+                                       W, K, K_bg_model, _ptr(v, _f32p), _ptr(vb, _f32p), C.byref(h)))
+        self.h = h
+
+    def hits_page(self, posset, p_cutoff, n_pos_sequences, cursor=0, cap=1 << 20, subset=None):
+        """One bamm_scan_hits call: (structured array of HIT_DTYPE, next cursor)."""
+        sub = np.ascontiguousarray(subset, np.uint64) if subset is not None else None
+        out = np.zeros(int(cap), HIT_DTYPE)
+        cur, n = C.c_uint64(int(cursor)), C.c_uint64(0)
+        _check(load().bamm_scan_hits(self.h, posset.h, _ptr(sub, _u64p), len(sub) if sub is not None else 0, int(n_pos_sequences),
+                                     C.c_float(p_cutoff), C.byref(cur), out.ctypes.data_as(_vp), int(cap), C.byref(n)))
+        return out[:n.value], cur.value
+
+    def hits(self, posset, p_cutoff, n_pos_sequences=None, subset=None, cap=1 << 20):
+        """Every hit of posset[subset] (default: all sequences), fetched in pages of `cap`: a page with fewer than `cap` hits
+        is the last one. n_pos_sequences defaults to the number of scanned sequences."""
+        n_pos = (len(subset) if subset is not None else posset.nseq) if n_pos_sequences is None else n_pos_sequences
+        pages, cursor = [], 0
+        while True:
+            page, cursor = self.hits_page(posset, p_cutoff, n_pos, cursor, cap, subset)
+            pages.append(page)
+            if len(page) < cap:
+                return np.concatenate(pages)
+
+    def info(self):
+        """dict(negative_windows, neg_score_ms, sort_ms, hits_ms): see bamm_scan_info."""
+        n = C.c_uint64(0)
+        a, b, c = C.c_float(0), C.c_float(0), C.c_float(0)
+        _check(load().bamm_scan_info(self.h, C.byref(n), C.byref(a), C.byref(b), C.byref(c)))
+        return dict(negative_windows=int(n.value), neg_score_ms=a.value, sort_ms=b.value, hits_ms=c.value)
+
+    def close(self):
+        if self.h:
+            load().bamm_scan_destroy(self.h)
             self.h = None
 
     def __del__(self):

@@ -6,6 +6,7 @@
 #include "launch.h"
 #include "negatives.cuh"
 #include "stats.cuh"
+#include "scan.cuh"
 #include <cub/device/device_scan.cuh>
 #include "fasta.cuh"
 #include "mask.cuh"
@@ -575,3 +576,4 @@ extern "C" int bamm_seqset_count_kmers(bamm_seqset* s, int K, uint64_t* n_all) {
 #include "capi_negatives.inl"
 #include "capi_score.inl"
 #include "capi_fasta.inl"
+#include "capi_scan.inl"

@@ -141,20 +141,20 @@ template <typename T> void fitLength( std::vector<T>& v, size_t n ){
 
 }  // namespace
 
-void Global::init( int nargs, char* args[] ){
-    readArguments( nargs, args );
+void Global::init( int nargs, char* args[], bool scan ){
+    readArguments( nargs, args, scan );
     Alphabet::init( alphabetType.c_str() );
     // positive set first, then the (by default identical) negative file: the order fixes the rand() stream of the
     // N draws (reference: Global.cpp:105-106)
     posSequenceSet = new SequenceSet( posSequenceFilename, ss );
     negSequenceSet = new SequenceSet( negSequenceFilename, ss );
-    if( posSequenceSet->getSequences().size() < cvFold ){
+    if( posSequenceSet->getSequences().size() < ( scan ? 1 : cvFold ) ){
         std::cerr << "Error: Input sequences are too few for training! \n" << std::endl;
         exit( 1 );
     }
 }
 
-int Global::readArguments( int nargs, char* args[] ){
+int Global::readArguments( int nargs, char* args[], bool scan ){
     if( nargs < 3 ){
         std::cerr << "Error: Arguments are missing! \n" << std::endl;
         printHelp();
@@ -241,7 +241,7 @@ int Global::readArguments( int nargs, char* args[] ){
     opt.value( "", 'f', f );
 
     FDR = opt.present( "FDR" );
-    if( FDR ){
+    if( FDR || scan ){
         opt.value( "mFold", 'm', mFold );
         opt.value( "cvFold", 'n', cvFold );
         opt.value( "sOrder", 's', sOrder );
@@ -273,6 +273,10 @@ int Global::readArguments( int nargs, char* args[] ){
     }
     opt.value( "threads", 0, threads );
     ( void )ignored;
+    if( scan && ( EM || CGS || advanceEM || FDR || scoreSeqset ) ){
+        std::cerr << "Error: BaMMScan scores the given motifs; --EM, --CGS, --advanceEM, --FDR and --scoreSeqset are options of BaMMmotif." << std::endl;
+        exit( 1 );
+    }
 
     if( opt.leftovers() ){
         printHelp();

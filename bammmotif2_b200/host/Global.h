@@ -12,7 +12,9 @@
 
 class Global {
 public:
-    static void init( int nargs, char* args[] );
+    // scan: the options of BaMMScan (mainScan.cpp): -m/--mFold and -s/--sOrder without --FDR, no training or evaluation
+    // options, and a single input sequence is enough
+    static void init( int nargs, char* args[], bool scan = false );
     static void destruct();
     static void printHelp();
     static void printStat();
@@ -76,7 +78,7 @@ public:
     static size_t       threads;
 
 private:
-    static int  readArguments( int nargs, char* args[] );
+    static int  readArguments( int nargs, char* args[], bool scan );
 };
 
 #endif

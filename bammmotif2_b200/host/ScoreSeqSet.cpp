@@ -84,26 +84,60 @@ void ScoreSeqSet::printLogOdds(){
     }
 }
 
-// .occurrence (reference: ScoreSeqSet::write, src/seq_scoring/ScoreSeqSet.cpp:245-291)
+// BaMMScan: the negative window scores are computed and sorted on the device once for this motif, the positive windows are
+// scored and given their p-values there, and only the windows with p < pvalCutoff come back (in sequence order, window
+// ascending) - the same windows and values as calcLogOdds + calcPvalues + the filter of write()
+void ScoreSeqSet::scanOccurrences( const std::vector<Sequence*>& negSet, float pvalCutoff ){
+    const int W = static_cast<int>( motif_->getW() ), K = static_cast<int>( motif_->getK() );
+    std::vector<uint64_t> negIdx, posIdx;
+    bool negWhole = false, posWhole = false;
+    SequenceSet* neg = SequenceSet::commonSet( negSet, negIdx, &negWhole );
+    SequenceSet* pos = SequenceSet::commonSet( seqSet_, posIdx, &posWhole );
+    bamm_scan* scan = nullptr;
+    BAMM_CHECK( bamm_scan_create( neg->device(), negWhole ? nullptr : negIdx.data(), negSet.size(), W, K, static_cast<int>( bg_->getOrder() ),
+                                  motif_->flatV().data(), bg_->flatV().data(), &scan ) );
+    hits_.clear();
+    const uint64_t page = 1u << 20;
+    uint64_t cursor = 0, got = page;
+    while( got == page ){
+        const size_t have = hits_.size();
+        hits_.resize( have + page );
+        BAMM_CHECK( bamm_scan_hits( scan, pos->device(), posWhole ? nullptr : posIdx.data(), seqSet_.size(), seqSet_.size(), pvalCutoff,
+                                    &cursor, hits_.data() + have, page, &got ) );
+        hits_.resize( have + got );
+    }
+    bamm_scan_destroy( scan );
+    hits_are_scanned_ = true;
+}
+
+// one line of the .occurrence file: window i of sequence n (reference: ScoreSeqSet.cpp:245-291)
+void ScoreSeqSet::writeOccurrence( std::ostream& ofile, size_t n, size_t i, float p, float e, bool ss ){
+    size_t seqlen = seqSet_[n]->getL();
+    if( !ss ) seqlen = ( seqlen - 1 ) / 2;
+    const size_t end = i + motif_->getW();
+    const uint8_t* codes = seqSet_[n]->getSequence();
+    ofile << seqSet_[n]->getHeader() << '\t' << seqlen << '\t' << ( ( i < seqlen ) ? '+' : '-' ) << '\t'
+          << i + 1 << ".." << end << '\t';
+    for( size_t m = i; m < end; m++ ) ofile << Alphabet::getBase( codes[m] );
+    ofile << '\t' << std::setprecision( 3 ) << p << '\t' << e << '\n';
+}
+
+// .occurrence (reference: ScoreSeqSet::write, src/seq_scoring/ScoreSeqSet.cpp:245-291): from the p-values of calcPvalues, or
+// from the hits of scanOccurrences
 void ScoreSeqSet::write( char* odir, std::string basename, float pvalCutoff, bool ss ){
-    assert( pval_is_calulated_ );
+    assert( pval_is_calulated_ || hits_are_scanned_ );
     std::ofstream ofile( std::string( odir ) + '/' + basename + ".occurrence" );
     ofile << "seq\tlength\tstrand\tstart..end\tpattern\tp-value\te-value" << std::endl;
+    if( !pval_is_calulated_ ){
+        for( const bamm_hit& h : hits_ )
+            if( h.p_value < pvalCutoff ) writeOccurrence( ofile, h.seq, h.window, h.p_value, h.e_value, ss );
+        return;
+    }
     const size_t W = motif_->getW();
     for( size_t n = 0; n < seqSet_.size(); n++ ){
-        size_t seqlen = seqSet_[n]->getL();
-        if( !ss ) seqlen = ( seqlen - 1 ) / 2;
         const size_t LW1 = seqSet_[n]->getL() - W + 1;
-        const uint8_t* codes = seqSet_[n]->getSequence();
-        for( size_t i = 0; i < LW1; i++ ){
-            if( mops_p_values_[n][i] < pvalCutoff ){
-                const size_t end = i + W;
-                ofile << seqSet_[n]->getHeader() << '\t' << seqlen << '\t' << ( ( i < seqlen ) ? '+' : '-' ) << '\t'
-                      << i + 1 << ".." << end << '\t';
-                for( size_t m = i; m < end; m++ ) ofile << Alphabet::getBase( codes[m] );
-                ofile << '\t' << std::setprecision( 3 ) << mops_p_values_[n][i] << '\t' << mops_e_values_[n][i] << '\n';
-            }
-        }
+        for( size_t i = 0; i < LW1; i++ )
+            if( mops_p_values_[n][i] < pvalCutoff ) writeOccurrence( ofile, n, i, mops_p_values_[n][i], mops_e_values_[n][i], ss );
     }
 }
 

@@ -1,6 +1,7 @@
 // ScoreSeqSet — log-odds scoring of every window of a sequence list; host wrapper over bamm_score_logodds().
 // Public interface = the reference's (src/seq_scoring/ScoreSeqSet.h:24-37). MOPS scores (one per window) are kept
 // flat; setKeepMops(false) skips materialising them when only ZOOPS scores are consumed (FDR's default).
+// scanOccurrences() is the route of BaMMScan: the negative scores stay on the device and only the hits come back.
 #ifndef BAMM_HOST_SCORESEQSET_H_
 #define BAMM_HOST_SCORESEQSET_H_
 
@@ -18,6 +19,10 @@ public:
     void setKeepMops( bool keep )   { keepMops_ = keep; }
     void calcLogOdds();
     void calcPvalues( std::vector<std::vector<float>> pos_mops_scores, std::vector<float> neg_all_scores );
+    // the windows with p < pvalCutoff, p against every window of negSet, all on the device (bamm_scan_*); write() then
+    // writes these hits
+    void scanOccurrences( const std::vector<Sequence*>& negSet, float pvalCutoff );
+    const std::vector<bamm_hit>&    getHits() const     { return hits_; }
 
     std::vector<std::vector<float>> getMopsScores();
     std::vector<float>              getZoopsScores()    { return zoops_scores_; }
@@ -29,6 +34,8 @@ public:
     void printLogOdds();
 
 private:
+    void writeOccurrence( std::ostream& out, size_t n, size_t i, float p, float e, bool ss );
+
     Motif*                          motif_;
     BackgroundModel*                bg_;
     std::vector<Sequence*>          seqSet_;
@@ -41,6 +48,8 @@ private:
     std::vector<std::vector<float>> mops_e_values_;
     std::vector<size_t>             z_;
     bool                            pval_is_calulated_ = false;
+    std::vector<bamm_hit>           hits_;
+    bool                            hits_are_scanned_ = false;
     std::vector<size_t>             Y_;
 };
 

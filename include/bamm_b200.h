@@ -285,6 +285,38 @@ int bamm_mops_pvalues(const float* neg_scores, uint64_t nneg, const float* pos_s
 /* device time (CUDA events on the scoring stream) of the scoring kernels of the last bamm_score_logodds call of this thread */
 int bamm_score_last_timing(float* kernel_ms);
 
+/* ---- occurrence scan  (BaMMScan: ScoreSeqSet::calcLogOdds + calcPvalues + the p < cutoff filter of ScoreSeqSet::write,
+ *      src/seq_scoring/ScoreSeqSet.cpp:25-67, 70-126, 245-291, with only the hits leaving the device) ------------------------ */
+/*
+ * A scan object holds one motif's log-odds table and the sorted scores of every window of its negative set, so that any
+ * number of positive sets (or parts of one) can be scanned against them. A hit is a positive window whose p-value (the
+ * formula of bamm_mops_pvalues, against ALL negative windows) is < p_cutoff (strict). Scores, p and e are the same bits as
+ * bamm_score_logodds(mops) + bamm_mops_pvalues give on the same inputs, and the hits come in the same order: subset order,
+ * then window ascending.
+ *   bamm_scan_create : scores the windows of neg[neg_subset] (NULL = all sequences) and sorts them, on the device. Fails
+ *                      with BAMM_E_NOMEM, naming the size, when the device cannot hold 8 bytes per negative window plus
+ *                      the sort's workspace. Inputs as bamm_score_logodds; an empty negative set is rejected.
+ *   bamm_scan_hits   : scans the windows of pos[subset] (NULL = all) from *cursor (0 = start) and writes at most `cap`
+ *                      hits; *nhits = hits written, *cursor = where the next call continues (the total number of windows
+ *                      of the subset when the scan is complete). `seq` of a hit is its index into `subset`, `window` its
+ *                      start. e = p * n_pos_sequences. pos must have the alphabet of the negative set.
+ */
+typedef struct bamm_scan bamm_scan;
+typedef struct bamm_hit {
+    uint64_t seq;         /* index into the subset */
+    uint64_t window;      /* window start in the stored sequence */
+    float    score, p_value, e_value;
+    uint32_t reserved;    /* 0 */
+} bamm_hit;
+int  bamm_scan_create(bamm_seqset* neg, const uint64_t* neg_subset, uint64_t nneg, int W, int K, int K_bg_model,
+                      const float* v_all, const float* vbg_all, bamm_scan** out);
+int  bamm_scan_hits(bamm_scan* sc, bamm_seqset* pos, const uint64_t* subset, uint64_t nsub, uint64_t n_pos_sequences,
+                    float p_cutoff, uint64_t* cursor, bamm_hit* hits, uint64_t cap, uint64_t* nhits);
+/* negative windows of the object, and the device times (CUDA events) of its negative scoring, of its sort, and of the
+ * kernels of the last bamm_scan_hits call (scoring with p-values, and hit compaction, summed over its chunks) */
+int  bamm_scan_info(bamm_scan* sc, uint64_t* n_negative_windows, float* neg_score_ms, float* sort_ms, float* hits_ms);
+void bamm_scan_destroy(bamm_scan* sc);
+
 #ifdef __cplusplus
 }
 #endif
