@@ -22,6 +22,7 @@
 #include <mutex>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 using namespace bamm;
@@ -119,6 +120,19 @@ static uint64_t ipow_u64(uint64_t b, int e) { uint64_t r = 1; while (e-- > 0) r 
 
 // ------------------------------------------------------------------------------------------- objects
 struct IndexArray { void* d = nullptr; int bytes = 2; uint64_t Yn = 0; };
+// The order-K index array holds uint16_t entries when A^(K+1) <= 65536 and uint32_t otherwise (seqset_index_locked); every
+// kernel that reads it is instantiated for both. f is a generic lambda and receives the typed pointer.
+template <typename F> static auto with_index(const IndexArray& ia, F&& f) { return ia.bytes == 2 ? f((const uint16_t*)ia.d) : f((const uint32_t*)ia.d); }
+template <typename F> static auto with_index_mut(IndexArray& ia, F&& f) { return ia.bytes == 2 ? f((uint16_t*)ia.d) : f((uint32_t*)ia.d); }
+// The column blocks of a W-column motif (column_blocks, kernels.cuh) as the compile-time NB of the index-array kernels
+template <typename F> static auto with_column_blocks(int W, F&& f) { return column_blocks(W) == 2 ? f(std::integral_constant<int, 2>()) : f(std::integral_constant<int, 1>()); }
+// Index-array kernels with the [j][y] table in shared memory run 512-thread CTAs, as many per SM as the opt-in shared memory
+// holds (1 KB per CTA reserved), at most 4 (2048 threads, the SM's limit); a table beyond shared memory: 4 CTAs per SM.
+struct TableGrid { bool smem; int grid; };
+static TableGrid table_grid(size_t table_bytes, int max_optin, int sms) {
+    if (table_bytes > (size_t)max_optin) return {false, sms * 4};
+    return {true, sms * std::max(1, std::min(4, (int)((size_t)(max_optin + 1024) / (table_bytes + 1024))))};
+}
 
 struct bamm_seqset {
     int device = 0;
@@ -477,15 +491,10 @@ static int seqset_index_locked(bamm_seqset* s, int K, IndexArray** out) {
     CU(dev_malloc(&ia.d, (s->npos ? s->npos : 1) * (uint64_t)ia.bytes));
     const int block = 256;
     const int grid = s->sm_count * 8;
-    if (s->nseq) {
-        if (ia.bytes == 2) k_build_index<uint16_t><<<grid, block>>>(s->d_codes, s->d_off, s->nseq, s->A, K, Yn, (uint16_t*)ia.d);
-        else               k_build_index<uint32_t><<<grid, block>>>(s->d_codes, s->d_off, s->nseq, s->A, K, Yn, (uint32_t*)ia.d);
-    }
-    if (s->npatch) {
-        const int pg = (int)((s->npatch + 255) / 256);
-        if (ia.bytes == 2) k_patch_index<uint16_t><<<pg, 256>>>(s->d_ppos, s->d_pkmer, s->npatch, Yn, (uint16_t*)ia.d);
-        else               k_patch_index<uint32_t><<<pg, 256>>>(s->d_ppos, s->d_pkmer, s->npatch, Yn, (uint32_t*)ia.d);
-    }
+    with_index_mut(ia, [&](auto Y) {
+        if (s->nseq) k_build_index<<<grid, block>>>(s->d_codes, s->d_off, s->nseq, s->A, K, Yn, Y);
+        if (s->npatch) k_patch_index<<<(int)((s->npatch + 255) / 256), 256>>>(s->d_ppos, s->d_pkmer, s->npatch, Yn, Y);
+    });
     cudaError_t e = cudaDeviceSynchronize();
     if (e == cudaSuccess) e = cudaGetLastError();
     if (e != cudaSuccess) { cudaFree(ia.d); return fail(BAMM_E_CUDA, "index build failed: %s", cudaGetErrorString(e)); }
@@ -546,13 +555,10 @@ extern "C" int bamm_seqset_count_kmers(bamm_seqset* s, int K, uint64_t* n_all) {
         const bool smem = ia->Yn <= 12288 && s->npos / ((uint64_t)s->sm_count * 8) < 0xffffffffull;     // 48 KB of 32-bit bins
         const size_t sh = smem ? (size_t)Yn * 4 : 0;
         const int grid = s->sm_count * 8;
-        if (ia->bytes == 2) {
-            if (smem) k_count_kmers<uint16_t, true><<<grid, 256, sh>>>((const uint16_t*)ia->d, s->npos, Yn, d_cnt);
-            else      k_count_kmers<uint16_t, false><<<grid, 256>>>((const uint16_t*)ia->d, s->npos, Yn, d_cnt);
-        } else {
-            if (smem) k_count_kmers<uint32_t, true><<<grid, 256, sh>>>((const uint32_t*)ia->d, s->npos, Yn, d_cnt);
-            else      k_count_kmers<uint32_t, false><<<grid, 256>>>((const uint32_t*)ia->d, s->npos, Yn, d_cnt);
-        }
+        with_index(*ia, [&](auto Y) {
+            using YT = std::decay_t<decltype(*Y)>;
+            (smem ? k_count_kmers<YT, true> : k_count_kmers<YT, false>)<<<grid, 256, sh>>>(Y, s->npos, Yn, d_cnt);
+        });
     }
     std::vector<uint64_t> top(ia->Yn);
     cudaError_t e = cudaMemcpy(top.data(), d_cnt, ia->Yn * 8, cudaMemcpyDeviceToHost);

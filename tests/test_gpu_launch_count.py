@@ -2,7 +2,8 @@
 call the count must move by the number of kernels torch.profiler's CUDA activity trace records during that call (copies and
 memsets are not kernels). Plans: c3's pruned E-step with bound reuse (two bound kernels per E-step); order 5 at W=20, pruned
 with column passes and dense with column passes (one launch per pass for the E-step kernels and the tables of every update);
-the six-letter alphabet (single-stranded) on the index-array row path."""
+the six-letter alphabet (single-stranded) on the index-array row path; order 8 (32-bit k-mer indices) on the row path with
+global count tables."""
 import json
 import os
 
@@ -16,7 +17,8 @@ _KEYS = ("BAMM_BOUND_REUSE", "BAMM_NO_BOUND_REUSE", "BAMM_BOUND_SLACK", "BAMM_WA
 PLANS = {"c3_40k_reuse": (4, 40000, 500, 20, 4, 2, {"BAMM_BOUND_REUSE": "1"}),
          "k5_w20_pruned": (4, 20000, 500, 20, 5, 2, {}),
          "k5_w20_dense": (4, 20000, 500, 20, 5, 2, {"BAMM_NO_SPARSE": "1"}),
-         "a6_rows": (6, 3000, 300, 12, 5, 2, {})}
+         "a6_rows": (6, 3000, 300, 12, 5, 2, {}),
+         "k8_rows_u32": (4, 3000, 300, 12, 8, 2, {})}
 
 
 @pytest.fixture(scope="module")

@@ -105,6 +105,7 @@ def em_against_oracle(capi, oracle, ss, kmer, offsets, A, K, W, v0, vbg, alpha, 
 
 @pytest.mark.parametrize("A,K,W", [(4, 0, 33), (4, 2, 40), (4, 3, 63), (4, 4, 48),      # table in shared memory
                                    (4, 4, 63), (4, 6, 36),                              # row-form E-step, k_mstep_cols
+                                   (4, 8, 12), (4, 8, 40),      # 32-bit k-mer indices: row-form E-step, global count tables
                                    (6, 2, 45), (6, 5, 36)])                             # EXTENDED alphabet
 def test_em_per_iteration_against_oracle(capi, oracle, A, K, W):
     ss, _, kmer, offsets = make_data(capi, oracle, A, W, 100 * A + K + W)
